@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- decoded audio-seconds/sec of the synthesis back-end, every BASELINE.json config in ONE line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline (`value`, `roofline`, `e2e`, `cpu_baseline`): BASELINE config 2 -- MP3 MPEG-1 44.1 kHz stereo, 8192 frames
 (64 streams x 128 consecutive frames) per GPU.  `value` is measured with inputs resident in HBM; `e2e` goes through the
@@ -22,6 +22,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -29,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: a benchmark run leaves it as it found it
 
 N_STREAMS = 64
 FRAMES_PER_STREAM = 128
@@ -82,12 +84,14 @@ class ClockSampler(threading.Thread):
 # ---- CPU arm: the oracle (C++ restatement of the reference's scalar path), built for THIS box ---------------------------
 
 def _load_oracle_native():
-    """Builds oracle/ with -march=native ON THIS BOX (the CPU baseline must use this host's ISA)."""
+    """Builds oracle/ with -march=native ON THIS BOX (the CPU baseline must use this host's ISA), into a temporary
+    directory: the source tree may be read-only."""
     from tests import _oracle
-    out = os.path.join(ROOT, "oracle", "_build", "liboracle_native.so")
     try:
-        _oracle.build(arch="-march=native", out="_build/liboracle_native.so")
-        return _oracle.load(out), "-march=native"
+        with tempfile.TemporaryDirectory(prefix="symgpu-oracle-") as tmp:
+            out = os.path.join(tmp, "liboracle_native.so")
+            _oracle.build(arch="-march=native", out=out)
+            return _oracle.load(out), "-march=native"
     except Exception:
         return _oracle.load(), "-march=x86-64-v3"
 
@@ -129,6 +133,17 @@ def _cpu_aac(orc, units, tns, coeffs, runs, n_threads, min_seconds):
 def _cpu_vorbis(orc, wl, n_threads, min_seconds):
     from tests import _oracle
     return _repeat(lambda: _oracle.vorbis_batch(orc, wl, n_threads), min_seconds)
+
+
+def dump_outputs(out_dir, pcm):
+    """Writes the PCM of the last timed headline step as out_dir/mp3_pcm.npy: float32 (frames, 2, 1152) for a fixed
+    sample of half the batch's frames (seed 0, in frame order), 38 MB of its 75 MB.  The inputs and the number of steps
+    before it follow from the arguments alone, so two builds run with the same arguments can be compared word for word."""
+    import torch
+    frames = np.sort(np.random.default_rng(0).choice(pcm.shape[0], pcm.shape[0] // 2, replace=False))
+    sample = pcm[torch.from_numpy(frames).to(pcm.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "mp3_pcm.npy"), sample)
 
 
 def _vorbis_algo_bytes(wl):
@@ -365,6 +380,8 @@ def run_ours(args):
     t0 = time.perf_counter()
     avg_kernel_ms, total_ms = time_device(step, args.steps, args.warmup)
     wall = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:  # before the untimed launches below overwrite every buffer set
+        dump_outputs(args.dump_outputs, sets[(args.warmup + args.steps - 1) % N_BUFFER_SETS][2])
     launches = eng.launch_count - launches0 - args.warmup
     # The clock sampler polls nvidia-smi (a few hundred ms per query, and its driver calls stall CUDA API calls for tens of
     # ms): it covers the device-timed region above and is stopped before the host-timed regions below.  A short timed
@@ -617,7 +634,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="only the MP3 headline (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the PCM of the last timed headline step (rank 0) as DIR/mp3_pcm.npy, a seeded half of its frames")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
