@@ -393,6 +393,15 @@ symgpu_status symgpu_pcm_pack_dev(symgpu_ctx* ctx, const float* pcm, const symgp
 symgpu_status symgpu_pcm_pack_host(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans,
                                    uint32_t n_spans, uint32_t channels, uint32_t plane_stride, uint32_t frames,
                                    int format, void* out, size_t out_bytes);
+/* The same with a channel map: output channel c reads plane plane_of_channel[c] (< channels; host memory in both variants), i.e.
+ * out[(dst_frame + i) * channels + c] = convert(pcm[src + plane_of_channel[c] * plane_stride + trim_start + i]).  With the identity
+ * map the output equals symgpu_pcm_pack_*. */
+symgpu_status symgpu_pcm_pack_mapped_dev(symgpu_ctx* ctx, const float* pcm, const symgpu_pcm_span* spans, uint32_t n_spans,
+                                         uint32_t channels, uint32_t plane_stride, uint32_t frames, const uint8_t* plane_of_channel,
+                                         int format, void* out);
+symgpu_status symgpu_pcm_pack_mapped_host(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans,
+                                          uint32_t n_spans, uint32_t channels, uint32_t plane_stride, uint32_t frames,
+                                          const uint8_t* plane_of_channel, int format, void* out, size_t out_bytes);
 
 /* symgpu_mp3_synth_host with the output stage in the pipeline: the stereo PCM of frame f is written to
  * out as interleaved samples [f * 1152 .. f * 1152 + 1152) of `format` (no trim); only the packed
@@ -764,8 +773,16 @@ symgpu_status symgpu_flac_index(const uint8_t* data, size_t n, symgpu_flac_strea
  *   Floor1::read_channel                                     floor.rs:655-722
  *   Residue::read_residue (types 0, 1, 2)                    residue.rs:142-543
  *   VorbisDecoder::decode_inner up to inverse coupling       lib.rs:146-250
- * What the synthesis kernel supports bounds what this accepts: 1 or 2 channels, floor type 1, at most one coupling step
- * (magnitude = channel 0, angle = channel 1); anything else is SYMGPU_ERR_UNSUPPORTED at create time.
+ * Two ways to open a stream, both refusing floor type 0 and setups symgpu_vorbis_floors_check refuses (SYMGPU_ERR_UNSUPPORTED):
+ *   symgpu_vorbis_fe_create     what symgpu_vorbis_synth_* takes: 1 or 2 channels, every mapping uncoupled or coupled by the one
+ *                               step (magnitude 0, angle 1), the same number of steps in every mode's mapping.  Used with the
+ *                               two-plane entry points (config, decode, decode_packets, decode_packets_jobs).
+ *   symgpu_vorbis_fe_create_mc  what symgpu_vorbis_mc_synth_* takes: 1 to 8 channels (more: SYMGPU_ERR_UNSUPPORTED, the reference has
+ *                               no channel map for them; 0: SYMGPU_ERR_DECODE), up to SYMGPU_VORBIS_MAX_COUPLINGS steps per mapping,
+ *                               every mode's mapping with the same coupling list.  Used with the *_mc entry points, which write
+ *                               `planes` channel planes (stream channels <= planes <= 8: streams of different channel counts can
+ *                               share one batch; planes beyond the stream's are zero, not decoded, without a floor).
+ * A front-end from create_mc takes the two-plane entry points only if create would have accepted the stream (else SYMGPU_ERR_ARG).
  * ================================================================================================= */
 typedef struct symgpu_vorbis_fe symgpu_vorbis_fe;
 /* ident: the 30-byte identification packet; setup: the setup packet (together: the stream's extra data). */
@@ -791,6 +808,23 @@ symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ident, size_t 
 symgpu_status symgpu_vorbis_fe_decode_packets(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets,
                                               uint32_t slot, uint32_t floor_base, symgpu_vorbis_unit* units, uint16_t* floor_y, float* residue,
                                               uint32_t* packet_of, size_t* n_good);
+/* The multichannel forms: records of symgpu_vorbis_mc_streams_set (couplings in mapping order) / _floors_set; per packet a
+ * symgpu_vorbis_unit_mc, floor_y [planes][65], residue [planes][slot] (packet k of a batch at 65 * planes * k / planes * slot * k). */
+symgpu_status symgpu_vorbis_fe_create_mc(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out);
+symgpu_status symgpu_vorbis_fe_config_mc(const symgpu_vorbis_fe* fe, symgpu_vorbis_stream_mc* stream, symgpu_vorbis_floor1* floors, uint32_t* n_floors);
+symgpu_status symgpu_vorbis_fe_decode_mc(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base, uint32_t planes,
+                                         symgpu_vorbis_unit_mc* unit, uint16_t* floor_y, float* residue);
+symgpu_status symgpu_vorbis_fe_decode_packets_mc(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets,
+                                                 uint32_t slot, uint32_t floor_base, uint32_t planes, symgpu_vorbis_unit_mc* units, uint16_t* floor_y,
+                                                 float* residue, uint32_t* packet_of, size_t* n_good);
+symgpu_status symgpu_vorbis_fe_decode_packets_jobs_mc(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, const uint8_t* data,
+                                                      size_t n, const symgpu_piece* packets, size_t n_packets, uint32_t slot, uint32_t floor_base,
+                                                      uint32_t planes, symgpu_vorbis_unit_mc* units, uint16_t* floor_y, float* residue, uint32_t* accepted,
+                                                      size_t* n_good, uint32_t n_threads);
+/* The reference's channel order (map_vorbis_channel, lib.rs:771-788; Vorbis I 4.3.9): Vorbis channel i of a `channels`-channel
+ * stream is output plane plane_of_channel[i].  symgpu_vorbis_*_synth_* write planes in Vorbis order; symgpu_pcm_pack_mapped_* with
+ * the inverse permutation produces the reference's order.  channels 1..8, else SYMGPU_ERR_ARG. */
+symgpu_status symgpu_vorbis_channel_map(uint32_t channels, uint8_t* plane_of_channel);
 
 /* ===================================================================================================
  * AAC-LC entropy front-end (SURVEY 8f N1): one raw_data_block per packet (an ADTS frame's payload, or an MP4 sample) ->

@@ -84,7 +84,7 @@ struct Packet { // PacketRef
 // Borrow of the decoder-owned planar f32 buffer, valid until the next call on the decoder
 // (GenericAudioBufferRef over AudioBuffer<f32>, symphonia-core/src/audio/buf.rs:68-73).
 struct AudioBufferRef {
-    const float* planes[2] = {nullptr, nullptr};
+    const float* planes[8] = {};  // n_planes of them, in the reference's channel order
     size_t n_planes = 0;
     size_t frames = 0;
 };
@@ -386,16 +386,26 @@ class GpuVorbisDecoder final : public AudioDecoder {
                                                          const AudioDecoderOptions& o) {
         if (p.codec != CODEC_ID_VORBIS) return {nullptr, {ErrorKind::Unsupported, "vorbis: invalid codec type"}};
         if (p.extra_data.size() <= 30) return {nullptr, {ErrorKind::Unsupported, "vorbis: missing extra data"}};
+        // a stream the two-plane front-end takes keeps that path; any other (3 to 8 channels, other couplings) opens multichannel
         symgpu_vorbis_fe* fe = nullptr;
-        symgpu_status st = symgpu_vorbis_fe_create(p.extra_data.data(), 30, p.extra_data.data() + 30, p.extra_data.size() - 30, &fe);
+        const uint8_t *ident = p.extra_data.data(), *setup = ident + 30;
+        symgpu_status st = symgpu_vorbis_fe_create(ident, 30, setup, p.extra_data.size() - 30, &fe);
+        const bool mc = st == SYMGPU_ERR_UNSUPPORTED;
+        if (mc) st = symgpu_vorbis_fe_create_mc(ident, 30, setup, p.extra_data.size() - 30, &fe);
         if (st != SYMGPU_OK) return {nullptr, map_status(st)};
         symgpu_vorbis_stream stream{};
+        symgpu_vorbis_stream_mc stream_mc{};
         std::vector<symgpu_vorbis_floor1> floors(64);
         uint32_t n_floors = 0;
-        symgpu_vorbis_fe_config(fe, &stream, floors.data(), &n_floors);
+        if (mc) {
+            symgpu_vorbis_fe_config_mc(fe, &stream_mc, floors.data(), &n_floors);
+            stream = symgpu_vorbis_stream{stream_mc.bs0_exp, stream_mc.bs1_exp, stream_mc.channels, 0};
+        } else {
+            symgpu_vorbis_fe_config(fe, &stream, floors.data(), &n_floors);
+        }
         symgpu_ctx* ctx = nullptr;
         st = symgpu_ctx_create(gpu->device(), &ctx);
-        if (st == SYMGPU_OK) st = symgpu_vorbis_streams_set(ctx, &stream, 1);
+        if (st == SYMGPU_OK) st = mc ? symgpu_vorbis_mc_streams_set(ctx, &stream_mc, 1) : symgpu_vorbis_streams_set(ctx, &stream, 1);
         if (st == SYMGPU_OK && n_floors) st = symgpu_vorbis_floors_set(ctx, floors.data(), n_floors);
         if (st != SYMGPU_OK) {
             symgpu_vorbis_fe_destroy(fe);
@@ -404,14 +414,15 @@ class GpuVorbisDecoder final : public AudioDecoder {
         }
         AudioCodecParameters params = p;
         params.channels = stream.channels;
-        return {std::unique_ptr<AudioDecoder>(new GpuVorbisDecoder(ctx, std::move(params), o, fe, stream)), {}};
+        return {std::unique_ptr<AudioDecoder>(new GpuVorbisDecoder(ctx, std::move(params), o, fe, stream, mc)), {}};
     }
     ~GpuVorbisDecoder() override {
         symgpu_vorbis_fe_destroy(fe_);
         symgpu_ctx_destroy(ctx_);
     }
     void reset() override {  // lib.rs:336-338 -> dsp.rs:26-32: overlap cleared, no previous block
-        symgpu_vorbis_stream_reset(ctx_, 0);
+        if (mc_) symgpu_vorbis_mc_stream_reset(ctx_, 0);
+        else symgpu_vorbis_stream_reset(ctx_, 0);
         symgpu_vorbis_fe_reset(fe_);
         have_prev_ = false;
         frames_ = 0;
@@ -419,12 +430,22 @@ class GpuVorbisDecoder final : public AudioDecoder {
     const AudioCodecParameters& codec_params() const override { return params_; }
     Result<AudioBufferRef> decode(const Packet& packet) override {
         frames_ = first_ = 0;
-        symgpu_vorbis_unit unit;
-        symgpu_status st = symgpu_vorbis_fe_decode(fe_, packet.data, packet.len, slot_, 0, &unit, floor_y_, residue_.data());
-        if (st != SYMGPU_OK) return {{}, map_status(st)};
         symgpu_vorbis_run run{};
         run.stream = 0, run.first_packet = 0, run.n_packets = 1;
-        st = symgpu_vorbis_synth_host(ctx_, &unit, floor_y_, residue_.data(), &run, 1, 1, slot_, pcm_.data());
+        symgpu_vorbis_unit_mc unit;  // (block flags only, in both paths)
+        symgpu_status st;
+        if (mc_) {
+            const uint32_t C = stream_.channels;
+            st = symgpu_vorbis_fe_decode_mc(fe_, packet.data, packet.len, slot_, 0, C, &unit, floor_y_, residue_.data());
+            if (st != SYMGPU_OK) return {{}, map_status(st)};
+            st = symgpu_vorbis_mc_synth_host(ctx_, &unit, floor_y_, residue_.data(), &run, 1, 1, C, slot_, pcm_.data());
+        } else {
+            symgpu_vorbis_unit u2;
+            st = symgpu_vorbis_fe_decode(fe_, packet.data, packet.len, slot_, 0, &u2, floor_y_, residue_.data());
+            if (st != SYMGPU_OK) return {{}, map_status(st)};
+            unit.block_flag = u2.block_flag, unit.prev_block_flag = u2.prev_block_flag;
+            st = symgpu_vorbis_synth_host(ctx_, &u2, floor_y_, residue_.data(), &run, 1, 1, slot_, pcm_.data());
+        }
         if (st != SYMGPU_OK) return {{}, map_status(st)};
         const size_t prev_n = size_t(1) << (unit.prev_block_flag ? stream_.bs1_exp : stream_.bs0_exp);
         const size_t n = size_t(1) << (unit.block_flag ? stream_.bs1_exp : stream_.bs0_exp);
@@ -445,22 +466,30 @@ class GpuVorbisDecoder final : public AudioDecoder {
         AudioBufferRef r;
         r.n_planes = params_.channels;
         r.frames = frames_;
-        r.planes[0] = pcm_.data() + first_;
-        r.planes[1] = pcm_.data() + slot_ + first_;
+        if (!mc_) {
+            r.planes[0] = pcm_.data() + first_;
+            r.planes[1] = pcm_.data() + slot_ + first_;
+            return r;
+        }
+        for (size_t i = 0; i < params_.channels; ++i) r.planes[map_[i]] = pcm_.data() + i * slot_ + first_;  // lib.rs:307-315
         return r;
     }
 
   private:
-    GpuVorbisDecoder(symgpu_ctx* ctx, AudioCodecParameters p, AudioDecoderOptions o, symgpu_vorbis_fe* fe, symgpu_vorbis_stream stream)
-        : ctx_(ctx), params_(std::move(p)), opts_(o), fe_(fe), stream_(stream), slot_((1u << stream.bs1_exp) >> 1),
-          residue_(2 * size_t(slot_), 0.0f), pcm_(2 * size_t(slot_), 0.0f) {}
+    GpuVorbisDecoder(symgpu_ctx* ctx, AudioCodecParameters p, AudioDecoderOptions o, symgpu_vorbis_fe* fe, symgpu_vorbis_stream stream, bool mc)
+        : ctx_(ctx), params_(std::move(p)), opts_(o), fe_(fe), stream_(stream), mc_(mc), slot_((1u << stream.bs1_exp) >> 1),
+          residue_(std::max<size_t>(2, stream.channels) * slot_, 0.0f), pcm_(std::max<size_t>(2, stream.channels) * slot_, 0.0f) {
+        symgpu_vorbis_channel_map(stream.channels, map_);
+    }
     symgpu_ctx* ctx_;
     AudioCodecParameters params_;
     AudioDecoderOptions opts_;
     symgpu_vorbis_fe* fe_;
-    symgpu_vorbis_stream stream_;
+    symgpu_vorbis_stream stream_;  // (channels and block sizes; `coupled` unused on the multichannel path)
+    bool mc_;
     uint32_t slot_;
-    uint16_t floor_y_[2 * 65];
+    uint8_t map_[SYMGPU_VORBIS_MAX_CHANNELS] = {};
+    uint16_t floor_y_[SYMGPU_VORBIS_MAX_CHANNELS * 65];
     std::vector<float> residue_, pcm_;
     size_t frames_ = 0, first_ = 0;
     bool have_prev_ = false;

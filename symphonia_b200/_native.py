@@ -280,6 +280,22 @@ def lib():
     L.symgpu_aac_fe_decode_packets_jobs.argtypes = [u32, u32, vp, sz, vp, sz, u32, vp, vp, sz, vp, ctypes.POINTER(sz), u32]
     L.symgpu_vorbis_fe_decode_packets_jobs.restype = ctypes.c_int
     L.symgpu_vorbis_fe_decode_packets_jobs.argtypes = [vp, sz, vp, sz, vp, sz, vp, sz, u32, u32, vp, vp, vp, vp, ctypes.POINTER(sz), u32]
+    L.symgpu_vorbis_fe_create_mc.restype = ctypes.c_int
+    L.symgpu_vorbis_fe_create_mc.argtypes = [vp, sz, vp, sz, ctypes.POINTER(vp)]
+    L.symgpu_vorbis_fe_config_mc.restype = ctypes.c_int
+    L.symgpu_vorbis_fe_config_mc.argtypes = [vp, vp, vp, ctypes.POINTER(u32)]
+    L.symgpu_vorbis_fe_decode_mc.restype = ctypes.c_int
+    L.symgpu_vorbis_fe_decode_mc.argtypes = [vp, vp, sz, u32, u32, u32, vp, vp, vp]
+    L.symgpu_vorbis_fe_decode_packets_mc.restype = ctypes.c_int
+    L.symgpu_vorbis_fe_decode_packets_mc.argtypes = [vp, vp, sz, vp, sz, u32, u32, u32, vp, vp, vp, vp, ctypes.POINTER(sz)]
+    L.symgpu_vorbis_fe_decode_packets_jobs_mc.restype = ctypes.c_int
+    L.symgpu_vorbis_fe_decode_packets_jobs_mc.argtypes = [vp, sz, vp, sz, vp, sz, vp, sz, u32, u32, u32, vp, vp, vp, vp, ctypes.POINTER(sz), u32]
+    L.symgpu_vorbis_channel_map.restype = ctypes.c_int
+    L.symgpu_vorbis_channel_map.argtypes = [u32, vp]
+    L.symgpu_pcm_pack_mapped_dev.restype = ctypes.c_int
+    L.symgpu_pcm_pack_mapped_dev.argtypes = [vp, vp, vp, u32, u32, u32, u32, vp, ctypes.c_int, vp]
+    L.symgpu_pcm_pack_mapped_host.restype = ctypes.c_int
+    L.symgpu_pcm_pack_mapped_host.argtypes = [vp, vp, sz, vp, u32, u32, u32, u32, vp, ctypes.c_int, vp, sz]
     L.symgpu_aac_fe_tables.restype = None
     L.symgpu_aac_fe_tables.argtypes = [vp, vp, vp]
     _LIB = L

@@ -4,7 +4,8 @@
 // (buf.rs:469-476) and FromSample<f32> (audio/conv.rs:592-607) for a whole batch.  Pure streaming:
 // 4 bytes read per sample, 1-4 written; bound by HBM.  One CTA walks spans grid-stride; for stereo
 // spans whose source and destination are 16-byte aligned each thread converts four frames from two
-// float4 loads and writes them with one or two 16-byte stores, otherwise one frame per thread.
+// float4 loads and writes them with one or two 16-byte stores, otherwise one frame per thread.  The MAPPED instances read
+// output channel c from plane map(c) instead of plane c (symgpu_pcm_pack_mapped_*); the unmapped ones are unchanged by that.
 #include "pack_kernel.h"
 
 namespace symgpu {
@@ -64,12 +65,18 @@ struct alignas(sizeof(T) * 8) Vec8 { // four stereo frames
     T v[8];
 };
 
-template <int FMT>
+template <bool MAPPED>
+__device__ __forceinline__ uint32_t plane_of(uint32_t plane_map, uint32_t c) {
+    return MAPPED ? (plane_map >> (4 * c)) & 15u : c;
+}
+
+template <int FMT, bool MAPPED>
 __global__ void __launch_bounds__(256) pack_kernel(PackArgs a) {
     using C = Conv<FMT>;
     using T = typename C::T;
     T* __restrict__ out = static_cast<T*>(a.out);
     const float* __restrict__ pcm = a.pcm;
+    const uint32_t map = a.plane_map;
     for (uint32_t p = blockIdx.x; p < a.n_spans; p += gridDim.x) {
         uint64_t src, dst;
         uint32_t stride, kept;
@@ -87,8 +94,9 @@ __global__ void __launch_bounds__(256) pack_kernel(PackArgs a) {
             dst = (uint64_t)p * a.frames;
         }
         if (a.channels == 2 && ((src | stride | dst) & 3) == 0) {
-            const float4* p0 = reinterpret_cast<const float4*>(pcm + src);
-            const float4* p1 = reinterpret_cast<const float4*>(pcm + src + stride);
+            const uint64_t s0 = src + (uint64_t)plane_of<MAPPED>(map, 0) * stride, s1 = src + (uint64_t)plane_of<MAPPED>(map, 1) * stride;
+            const float4* p0 = reinterpret_cast<const float4*>(pcm + s0);
+            const float4* p1 = reinterpret_cast<const float4*>(pcm + s1);
             Vec8<T>* o = reinterpret_cast<Vec8<T>*>(out + dst * 2);
             const uint32_t quads = kept >> 2;
             for (uint32_t q = threadIdx.x; q < quads; q += blockDim.x) {
@@ -101,14 +109,16 @@ __global__ void __launch_bounds__(256) pack_kernel(PackArgs a) {
                 o[q] = w;
             }
             for (uint32_t i = (quads << 2) + threadIdx.x; i < kept; i += blockDim.x) {
-                out[(dst + i) * 2] = C::of(__ldg(pcm + src + i));
-                out[(dst + i) * 2 + 1] = C::of(__ldg(pcm + src + stride + i));
+                out[(dst + i) * 2] = C::of(__ldg(pcm + s0 + i));
+                out[(dst + i) * 2 + 1] = C::of(__ldg(pcm + s1 + i));
             }
         } else {
             const uint32_t ch = a.channels;
-            for (uint32_t i = threadIdx.x; i < kept; i += blockDim.x)
-                for (uint32_t c = 0; c < ch; ++c)
-                    out[(dst + i) * ch + c] = C::of(__ldg(pcm + src + (uint64_t)c * stride + i));
+            for (uint32_t i = threadIdx.x; i < kept; i += blockDim.x) {
+                uint32_t m = map; // (shifted per channel: indexing it by (4 * c) makes ptxas spill)
+                for (uint32_t c = 0; c < ch; ++c, m >>= 4)
+                    out[(dst + i) * ch + c] = C::of(__ldg(pcm + src + (uint64_t)(MAPPED ? m & 15u : c) * stride + i));
+            }
         }
     }
 }
@@ -144,7 +154,24 @@ cudaError_t dequant_launch(const int16_t* q, float* spectra, size_t n, const flo
     return cudaGetLastError();
 }
 
-cudaError_t pack_launch(const PackArgs& a, int format, cudaStream_t stream) {
+namespace {
+
+template <bool MAPPED>
+cudaError_t pack_launch_as(const PackArgs& a, int format, unsigned grid, cudaStream_t stream) {
+    switch (format) {
+    case SYMGPU_FMT_F32: pack_kernel<SYMGPU_FMT_F32, MAPPED><<<grid, 256, 0, stream>>>(a); break;
+    case SYMGPU_FMT_S16: pack_kernel<SYMGPU_FMT_S16, MAPPED><<<grid, 256, 0, stream>>>(a); break;
+    case SYMGPU_FMT_S24: pack_kernel<SYMGPU_FMT_S24, MAPPED><<<grid, 256, 0, stream>>>(a); break;
+    case SYMGPU_FMT_S32: pack_kernel<SYMGPU_FMT_S32, MAPPED><<<grid, 256, 0, stream>>>(a); break;
+    case SYMGPU_FMT_U8: pack_kernel<SYMGPU_FMT_U8, MAPPED><<<grid, 256, 0, stream>>>(a); break;
+    default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+} // namespace
+
+cudaError_t pack_launch(const PackArgs& a, int format, cudaStream_t stream, bool mapped) {
     if (a.n_spans == 0) return cudaSuccess;
     static int sms = 0;
     if (!sms) {
@@ -154,15 +181,7 @@ cudaError_t pack_launch(const PackArgs& a, int format, cudaStream_t stream) {
     }
     const unsigned cap = (unsigned)sms * 8;
     const unsigned grid = a.n_spans < cap ? a.n_spans : cap;
-    switch (format) {
-    case SYMGPU_FMT_F32: pack_kernel<SYMGPU_FMT_F32><<<grid, 256, 0, stream>>>(a); break;
-    case SYMGPU_FMT_S16: pack_kernel<SYMGPU_FMT_S16><<<grid, 256, 0, stream>>>(a); break;
-    case SYMGPU_FMT_S24: pack_kernel<SYMGPU_FMT_S24><<<grid, 256, 0, stream>>>(a); break;
-    case SYMGPU_FMT_S32: pack_kernel<SYMGPU_FMT_S32><<<grid, 256, 0, stream>>>(a); break;
-    case SYMGPU_FMT_U8: pack_kernel<SYMGPU_FMT_U8><<<grid, 256, 0, stream>>>(a); break;
-    default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return mapped ? pack_launch_as<true>(a, format, grid, stream) : pack_launch_as<false>(a, format, grid, stream);
 }
 
 } // namespace symgpu

@@ -16,9 +16,11 @@ struct PackArgs {
     uint32_t plane_stride;
     uint32_t frames;
     void* out;
+    uint32_t plane_map;           // with `mapped`: output channel c reads plane (plane_map >> 4c) & 15
 };
 
-cudaError_t pack_launch(const PackArgs& a, int format, cudaStream_t stream);
+// mapped = false: output channel c reads plane c (plane_map unused).
+cudaError_t pack_launch(const PackArgs& a, int format, cudaStream_t stream, bool mapped = false);
 // spectra[i] = sign(q[i]) * pow43[|q[i]|] for n values (n a multiple of 8, both pointers 16-byte aligned).
 cudaError_t dequant_launch(const int16_t* q, float* spectra, size_t n, const float* pow43, cudaStream_t stream);
 

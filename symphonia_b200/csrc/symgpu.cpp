@@ -1034,24 +1034,34 @@ size_t symgpu_sample_bytes(int format) {
     }
 }
 
-symgpu_status symgpu_pcm_pack_dev(symgpu_ctx* ctx, const float* pcm, const symgpu_pcm_span* spans, uint32_t n_spans,
-                                  uint32_t channels, uint32_t plane_stride, uint32_t frames, int format, void* out) {
+// map: nullptr, or the plane of every output channel (checked: < channels), packed into PackArgs::plane_map
+static symgpu_status pcm_pack_dev_impl(symgpu_ctx* ctx, const float* pcm, const symgpu_pcm_span* spans, uint32_t n_spans, uint32_t channels,
+                                       uint32_t plane_stride, uint32_t frames, const uint8_t* map, int format, void* out) {
     if (!ctx || !pcm || !out || channels == 0 || channels > 8) return SYMGPU_ERR_ARG;
     if (symgpu_sample_bytes(format) == 0) return SYMGPU_ERR_ARG;
+    uint32_t plane_map = 0;
+    if (map)
+        for (uint32_t c = 0; c < channels; ++c) {
+            if (map[c] >= channels) return SYMGPU_ERR_ARG;
+            plane_map |= (uint32_t)map[c] << (4 * c);
+        }
     if (n_spans == 0) return SYMGPU_OK;
     DeviceGuard guard(ctx->device);
-    symgpu::PackArgs pa{pcm, spans, n_spans, channels, plane_stride, frames, out};
-    CU(ctx, symgpu::pack_launch(pa, format, ctx->stream));
+    symgpu::PackArgs pa{pcm, spans, n_spans, channels, plane_stride, frames, out, plane_map};
+    CU(ctx, symgpu::pack_launch(pa, format, ctx->stream, map != nullptr));
     ctx->launches += 1;
     return SYMGPU_OK;
 }
 
-symgpu_status symgpu_pcm_pack_host(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans,
-                                   uint32_t n_spans, uint32_t channels, uint32_t plane_stride, uint32_t frames,
-                                   int format, void* out, size_t out_bytes) {
+static symgpu_status pcm_pack_host_impl(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans, uint32_t n_spans,
+                                        uint32_t channels, uint32_t plane_stride, uint32_t frames, const uint8_t* map, int format, void* out,
+                                        size_t out_bytes) {
     if (!ctx || !pcm || !out || channels == 0 || channels > 8) return SYMGPU_ERR_ARG;
     const size_t sb = symgpu_sample_bytes(format);
     if (sb == 0) return SYMGPU_ERR_ARG;
+    if (map)
+        for (uint32_t c = 0; c < channels; ++c)
+            if (map[c] >= channels) return SYMGPU_ERR_ARG;
     if (n_spans == 0) return SYMGPU_OK;
     // Every span must stay inside the buffers the caller described.
     for (uint32_t p = 0; p < n_spans; ++p) {
@@ -1073,13 +1083,37 @@ symgpu_status symgpu_pcm_pack_host(symgpu_ctx* ctx, const float* pcm, size_t pcm
     if (spans) CU(ctx, cudaMemcpyAsync(base + in_bytes, spans, (size_t)n_spans * sizeof(symgpu_pcm_span), cudaMemcpyHostToDevice, ctx->stream));
     // Samples no span writes keep the caller's bytes.
     CU(ctx, cudaMemcpyAsync(base + in_bytes + span_bytes, out, out_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    s = symgpu_pcm_pack_dev(ctx, reinterpret_cast<const float*>(base),
-                            spans ? reinterpret_cast<const symgpu_pcm_span*>(base + in_bytes) : nullptr, n_spans, channels,
-                            plane_stride, frames, format, base + in_bytes + span_bytes);
+    s = pcm_pack_dev_impl(ctx, reinterpret_cast<const float*>(base), spans ? reinterpret_cast<const symgpu_pcm_span*>(base + in_bytes) : nullptr,
+                          n_spans, channels, plane_stride, frames, map, format, base + in_bytes + span_bytes);
     if (s != SYMGPU_OK) return s;
     CU(ctx, cudaMemcpyAsync(out, base + in_bytes + span_bytes, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return SYMGPU_OK;
+}
+
+symgpu_status symgpu_pcm_pack_dev(symgpu_ctx* ctx, const float* pcm, const symgpu_pcm_span* spans, uint32_t n_spans,
+                                  uint32_t channels, uint32_t plane_stride, uint32_t frames, int format, void* out) {
+    return pcm_pack_dev_impl(ctx, pcm, spans, n_spans, channels, plane_stride, frames, nullptr, format, out);
+}
+
+symgpu_status symgpu_pcm_pack_host(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans,
+                                   uint32_t n_spans, uint32_t channels, uint32_t plane_stride, uint32_t frames,
+                                   int format, void* out, size_t out_bytes) {
+    return pcm_pack_host_impl(ctx, pcm, pcm_floats, spans, n_spans, channels, plane_stride, frames, nullptr, format, out, out_bytes);
+}
+
+symgpu_status symgpu_pcm_pack_mapped_dev(symgpu_ctx* ctx, const float* pcm, const symgpu_pcm_span* spans, uint32_t n_spans,
+                                         uint32_t channels, uint32_t plane_stride, uint32_t frames, const uint8_t* plane_of_channel,
+                                         int format, void* out) {
+    if (!plane_of_channel) return SYMGPU_ERR_ARG;
+    return pcm_pack_dev_impl(ctx, pcm, spans, n_spans, channels, plane_stride, frames, plane_of_channel, format, out);
+}
+
+symgpu_status symgpu_pcm_pack_mapped_host(symgpu_ctx* ctx, const float* pcm, size_t pcm_floats, const symgpu_pcm_span* spans,
+                                          uint32_t n_spans, uint32_t channels, uint32_t plane_stride, uint32_t frames,
+                                          const uint8_t* plane_of_channel, int format, void* out, size_t out_bytes) {
+    if (!plane_of_channel) return SYMGPU_ERR_ARG;
+    return pcm_pack_host_impl(ctx, pcm, pcm_floats, spans, n_spans, channels, plane_stride, frames, plane_of_channel, format, out, out_bytes);
 }
 
 // ---- MPEG Layer I / II ---------------------------------------------------------------------------------

@@ -1,7 +1,7 @@
 // Vorbis entropy front-end (include/symgpu.h "Vorbis entropy front-end", SURVEY §8f N1): codebooks, floor-1 packet
 // decode, residue decode and the packet-level bookkeeping of VorbisDecoder::decode_inner up to -- not including --
 // inverse coupling (symphonia-codec-vorbis/src/{codebook,floor,residue,lib}.rs).  Output: what symgpu_vorbis_synth_*
-// reads.  CPU only.
+// (two planes) or symgpu_vorbis_mc_synth_* (up to eight) reads.  CPU only.
 //
 // Floating point, bit-exact by construction: a VQ table value is `m * delta + min (+ last)` in f32 in that order, a
 // residue element the running f32 sum of the vectors laid over it in pass order -- the same single IEEE operations in
@@ -254,6 +254,7 @@ struct symgpu_vorbis_fe {
     VorbisIdent ident{};
     VorbisSetup setup;
     std::vector<Codebook> books;
+    bool stereo = false;                // what symgpu_vorbis_fe_create accepts: the two-plane entry points may decode it
     int prev_block_flag = -1;
     std::vector<float> type2;
     std::vector<uint8_t> part_classes;  // persistent across packets, see read_residue
@@ -324,7 +325,7 @@ bool read_partition(const Codebook& book, PacketBits& bs, float* out, size_t n, 
     return true;
 }
 
-// residue.rs:142-449 for the channels in `chans` (1 or 2 of them).  0 ok, 1 decode error.
+// residue.rs:142-449 for the channels in `chans` (1 to 8 of them).  0 ok, 1 decode error.
 int read_residue(symgpu_vorbis_fe& fe, const VorbisResidueSetup& r, PacketBits& bs, unsigned bs_exp, const int* chans, int n_chans,
                  const uint8_t* do_not_decode, float* residue, uint32_t slot) {
     const Codebook& class_book = fe.books[r.classbook];
@@ -334,7 +335,7 @@ int read_residue(symgpu_vorbis_fe& fe, const VorbisResidueSetup& r, PacketBits& 
     const size_t part_size = r.partition_size, per_word = class_book.dims, parts = (end - begin) / part_size;
     bool any = false;
     for (int c = 0; c < n_chans; ++c) any |= !do_not_decode[chans[c]];
-    float* target[2] = {nullptr, nullptr};
+    float* target[SYMGPU_VORBIS_MAX_CHANNELS] = {};
     if (r.type == 2) {
         fe.type2.assign(full, 0.0f);
     } else {
@@ -385,9 +386,13 @@ int read_residue(symgpu_vorbis_fe& fe, const VorbisResidueSetup& r, PacketBits& 
 
 }  // namespace
 
-extern "C" symgpu_status symgpu_vorbis_fe_create(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out) {
-    if (!ident || !setup || !out) return SYMGPU_ERR_ARG;
-    std::unique_ptr<symgpu_vorbis_fe> fe(new (std::nothrow) symgpu_vorbis_fe());
+namespace {
+
+// Headers -> front-end, with what both create entry points refuse.  Sets fe->stereo when the stream is one the two-plane synthesis
+// takes: at most two channels and every mapping uncoupled or coupled by the one step (0, 1), the same number of steps in every mode.
+symgpu_status open_stream(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, std::unique_ptr<symgpu_vorbis_fe>& fe) {
+    if (!ident || !setup) return SYMGPU_ERR_ARG;
+    fe.reset(new (std::nothrow) symgpu_vorbis_fe());
     if (!fe) return SYMGPU_ERR_LIMIT;
     const Status si = vorbis_read_ident(ident, n_ident, fe->ident);
     if (si != Status::Ok) return si == Status::Unsupported ? SYMGPU_ERR_UNSUPPORTED : SYMGPU_ERR_DECODE;
@@ -399,13 +404,15 @@ extern "C" symgpu_status symgpu_vorbis_fe_create(const uint8_t* ident, size_t n_
     for (uint32_t k = 0; k < n_books; ++k)
         if (read_codebook(bs, fe->books[k])) return SYMGPU_ERR_DECODE;
     // residue partitions must fit the blocks they are laid over (the reference would panic slicing past the vector)
-    // -- checked per packet; here: what the synthesis kernel cannot take
-    if (fe->ident.n_channels > 2) return SYMGPU_ERR_UNSUPPORTED;
+    // -- checked per packet; here: what the synthesis kernels cannot take.  The reference has no channel map beyond 8 (lib.rs:771-788).
+    if (fe->ident.n_channels > SYMGPU_VORBIS_MAX_CHANNELS) return SYMGPU_ERR_UNSUPPORTED;
     for (uint8_t t : fe->setup.floor_type)
         if (t != 1) return SYMGPU_ERR_UNSUPPORTED;
+    bool stereo = fe->ident.n_channels <= 2;
     for (const auto& m : fe->setup.mappings) {
-        if (m.couplings.size() > 1) return SYMGPU_ERR_UNSUPPORTED;
-        if (m.couplings.size() == 1 && !(m.couplings[0].first == 0 && m.couplings[0].second == 1)) return SYMGPU_ERR_UNSUPPORTED;
+        if (m.couplings.size() > SYMGPU_VORBIS_MAX_COUPLINGS) return SYMGPU_ERR_UNSUPPORTED;
+        if (m.couplings.size() > 1) stereo = false;
+        if (m.couplings.size() == 1 && !(m.couplings[0].first == 0 && m.couplings[0].second == 1)) stereo = false;
     }
     // what symgpu_vorbis_floors_set will insist on at launch time is refused here, per stream (a setup whose read X values
     // repeat an implied end point passes the reference's parser but would divide by zero in its render_line)
@@ -420,22 +427,20 @@ extern "C" symgpu_status symgpu_vorbis_fe_create(const uint8_t* ident, size_t n_
         }
         if (!fl.empty() && symgpu_vorbis_floors_check(fl.data(), uint32_t(fl.size())) != SYMGPU_OK) return SYMGPU_ERR_UNSUPPORTED;
     }
-    // one coupling flag per stream record: every mode's mapping must agree
-    for (size_t k = 1; k < fe->setup.modes.size(); ++k)
-        if (fe->setup.mappings[fe->setup.modes[k].second].couplings.size() != fe->setup.mappings[fe->setup.modes[0].second].couplings.size())
-            return SYMGPU_ERR_UNSUPPORTED;
-    *out = fe.release();
-    return SYMGPU_OK;
-}
-extern "C" void symgpu_vorbis_fe_destroy(symgpu_vorbis_fe* fe) { delete fe; }
-extern "C" void symgpu_vorbis_fe_reset(symgpu_vorbis_fe* fe) {
-    if (fe) fe->prev_block_flag = -1;
+    // one coupling record per stream: the two-plane record holds a flag (every mode's mapping must agree on the step count), the
+    // multichannel record a list (every mode's mapping must have the same list)
+    const auto& first = fe->setup.mappings[fe->setup.modes[0].second].couplings;
+    bool same_lists = true;
+    for (size_t k = 1; k < fe->setup.modes.size(); ++k) {
+        const auto& c = fe->setup.mappings[fe->setup.modes[k].second].couplings;
+        if (c.size() != first.size()) stereo = false;
+        if (c != first) same_lists = false;
+    }
+    fe->stereo = stereo;  // (implies same_lists)
+    return same_lists ? SYMGPU_OK : SYMGPU_ERR_UNSUPPORTED;
 }
 
-extern "C" symgpu_status symgpu_vorbis_fe_config(const symgpu_vorbis_fe* fe, symgpu_vorbis_stream* stream, symgpu_vorbis_floor1* floors, uint32_t* n_floors) {
-    if (!fe || !stream || !floors || !n_floors) return SYMGPU_ERR_ARG;
-    *stream = symgpu_vorbis_stream{fe->ident.bs0_exp, fe->ident.bs1_exp, fe->ident.n_channels,
-                                   uint8_t(fe->setup.mappings[fe->setup.modes[0].second].couplings.empty() ? 0 : 1)};
+void floor_records(const symgpu_vorbis_fe* fe, symgpu_vorbis_floor1* floors, uint32_t* n_floors) {
     *n_floors = uint32_t(fe->setup.floor1.size());
     for (size_t i = 0; i < fe->setup.floor1.size(); ++i) {
         const VorbisFloor1Setup& f = fe->setup.floor1[i];
@@ -444,13 +449,12 @@ extern "C" symgpu_status symgpu_vorbis_fe_config(const symgpu_vorbis_fe* fe, sym
         o.multiplier = f.multiplier, o.n_posts = f.n_posts;
         std::memcpy(o.x_list, f.x_list, sizeof o.x_list), std::memcpy(o.low, f.low, 65), std::memcpy(o.high, f.high, 65), std::memcpy(o.sort_order, f.sort_order, 65);
     }
-    return SYMGPU_OK;
 }
 
-extern "C" symgpu_status symgpu_vorbis_fe_decode(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base,
-                                                 symgpu_vorbis_unit* unit, uint16_t* floor_y, float* residue) {
-    if (!fe || (!packet && n) || !unit || !floor_y || !residue) return SYMGPU_ERR_ARG;
-    if (slot < ((1u << fe->ident.bs1_exp) >> 1)) return SYMGPU_ERR_ARG;
+// One audio packet into `planes` channel planes (floor_y [planes][65], residue [planes][slot]); the stereo and multichannel entry points
+// both come here.  Planes beyond the stream's channels are zero, marked not decoded and without a floor.
+symgpu_status decode_packet(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base, uint32_t planes,
+                            symgpu_vorbis_unit_mc* unit, uint16_t* floor_y, float* residue) {
     PacketBits bs(packet, n);
     bool flag;
     if (!bs.read_bool(flag) || flag) return SYMGPU_ERR_DECODE;  // lib.rs:151-154
@@ -465,11 +469,11 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode(symgpu_vorbis_fe* fe, const uin
     const unsigned bs_exp = long_block ? fe->ident.bs1_exp : fe->ident.bs0_exp;
     const int n_ch = fe->ident.n_channels;
     std::memset(unit, 0, sizeof *unit);
-    std::memset(floor_y, 0, sizeof(uint16_t) * 2 * 65);
-    std::memset(residue, 0, sizeof(float) * 2 * size_t(slot));
+    std::memset(floor_y, 0, sizeof(uint16_t) * planes * 65);
+    std::memset(residue, 0, sizeof(float) * planes * size_t(slot));
     unit->block_flag = long_block;
     unit->prev_block_flag = uint8_t(fe->prev_block_flag < 0 ? long_block : fe->prev_block_flag);
-    unit->floor[0] = unit->floor[1] = 0xffff, unit->do_not_decode[0] = unit->do_not_decode[1] = 1;
+    for (int ch = 0; ch < SYMGPU_VORBIS_MAX_CHANNELS; ++ch) unit->floor[ch] = 0xffff, unit->do_not_decode[ch] = 1;
     // floors, one per channel (lib.rs:184-207).  A packet that ends inside a floor leaves that floor unused and everything
     // behind it unread -- which the reader reports by failing every later read, exactly the reference's behaviour.
     for (int ch = 0; ch < n_ch; ++ch) {
@@ -480,12 +484,12 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode(symgpu_vorbis_fe* fe, const uin
         unit->floor[ch] = used ? uint16_t(floor_base + floor_idx) : uint16_t(0xffff);
         if (!used) std::memset(floor_y + ch * 65, 0, sizeof(uint16_t) * 65);
     }
-    // non-zero vector propagate (lib.rs:213-225)
+    // non-zero vector propagate (lib.rs:213-225), step by step in mapping order
     for (const auto& cp : mapping.couplings)
         if (unit->do_not_decode[cp.first] != unit->do_not_decode[cp.second]) unit->do_not_decode[cp.first] = unit->do_not_decode[cp.second] = 0;
     // residues, per sub-map (lib.rs:229-248)
     for (int sm = 0; sm < mapping.n_submaps; ++sm) {
-        int chans[2], n_chans = 0;
+        int chans[SYMGPU_VORBIS_MAX_CHANNELS], n_chans = 0;
         for (int ch = 0; ch < n_ch; ++ch)
             if (mapping.multiplex[ch] == sm) chans[n_chans++] = ch;
         const VorbisResidueSetup& r = fe->setup.residues[mapping.submap_residue[sm]];
@@ -501,16 +505,33 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode(symgpu_vorbis_fe* fe, const uin
     return SYMGPU_OK;
 }
 
-extern "C" symgpu_status symgpu_vorbis_fe_decode_packets(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets,
-                                                         uint32_t slot, uint32_t floor_base, symgpu_vorbis_unit* units, uint16_t* floor_y, float* residue,
-                                                         uint32_t* packet_of, size_t* n_good) {
+// the two record layouts of a decoded packet
+constexpr uint32_t planes_of(const symgpu_vorbis_unit*) { return 2; }
+symgpu_status decode_into(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base, uint32_t,
+                          symgpu_vorbis_unit* unit, uint16_t* floor_y, float* residue) {
+    return symgpu_vorbis_fe_decode(fe, packet, n, slot, floor_base, unit, floor_y, residue);
+}
+symgpu_status decode_into(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base, uint32_t planes,
+                          symgpu_vorbis_unit_mc* unit, uint16_t* floor_y, float* residue) {
+    return symgpu_vorbis_fe_decode_mc(fe, packet, n, slot, floor_base, planes, unit, floor_y, residue);
+}
+symgpu_status create_for(const symgpu_vorbis_unit*, const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out) {
+    return symgpu_vorbis_fe_create(ident, n_ident, setup, n_setup, out);
+}
+symgpu_status create_for(const symgpu_vorbis_unit_mc*, const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out) {
+    return symgpu_vorbis_fe_create_mc(ident, n_ident, setup, n_setup, out);
+}
+
+template <class Unit>
+symgpu_status decode_packets(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets, uint32_t slot,
+                             uint32_t floor_base, uint32_t planes, Unit* units, uint16_t* floor_y, float* residue, uint32_t* packet_of, size_t* n_good) {
     if (!fe || (!data && n) || (n_packets && (!packets || !units || !floor_y || !residue || !packet_of)) || !n_good) return SYMGPU_ERR_ARG;
     if (slot < ((1u << fe->ident.bs1_exp) >> 1)) return SYMGPU_ERR_ARG;
     size_t good = 0;
     for (size_t i = 0; i < n_packets; ++i) {
         if (packets[i].offset > n || packets[i].len > n - packets[i].offset) continue;
-        const symgpu_status st = symgpu_vorbis_fe_decode(fe, data + packets[i].offset, packets[i].len, slot, floor_base, units + good, floor_y + 130 * good,
-                                                         residue + 2 * size_t(slot) * good);
+        const symgpu_status st = decode_into(fe, data + packets[i].offset, packets[i].len, slot, floor_base, planes, units + good,
+                                             floor_y + 65 * size_t(planes) * good, residue + size_t(planes) * slot * good);
         if (st != SYMGPU_OK) continue;  // the caller of the reference drops the packet and goes on
         packet_of[good++] = uint32_t(i);
     }
@@ -521,13 +542,16 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode_packets(symgpu_vorbis_fe* fe, c
 // A stream's audio packets as independent jobs (DESIGN 10.9): a packet depends on its predecessors only through the previous block
 // flag, which is output, not input, of the entropy stage -- the partition-class vector's history never reaches an entry a packet reads
 // before writing it, and what a class word writes does not depend on the vector's length beyond the entries it has (the digits kept
-// when it is cut are the same most significant ones).  Every thread owns a front-end built from the headers; outputs stay at their
-// packet's index (units[i], floor_y[130 i], residue[2 slot i]); accepted[0 .. n_good) lists the packets the reference decodes, in
-// order, and the previous block flags are chained over exactly those.
-extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, const uint8_t* data,
-                                                              size_t n, const symgpu_piece* packets, size_t n_packets, uint32_t slot, uint32_t floor_base,
-                                                              symgpu_vorbis_unit* units, uint16_t* floor_y, float* residue, uint32_t* accepted, size_t* n_good,
-                                                              uint32_t n_threads) {
+// when it is cut are the same most significant ones).  This holds for any number of channels per sub-map: a residue's pass 0 writes the
+// class words of every decoded channel of a partition group before any entry of that group is read, a channel only reads its own
+// entries [c * parts, (c + 1) * parts), and the vector is at least parts * channels long, so those entries are never cut; what an
+// earlier channel's last word spills into them is written in the same packet.  Every thread owns a front-end built from the headers;
+// outputs stay at their packet's index (units[i], floor_y[65 planes i], residue[planes slot i]); accepted[0 .. n_good) lists the
+// packets the reference decodes, in order, and the previous block flags are chained over exactly those.
+template <class Unit>
+symgpu_status decode_packets_jobs(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, const uint8_t* data, size_t n,
+                                  const symgpu_piece* packets, size_t n_packets, uint32_t slot, uint32_t floor_base, uint32_t planes, Unit* units,
+                                  uint16_t* floor_y, float* residue, uint32_t* accepted, size_t* n_good, uint32_t n_threads) {
     if (n_good) *n_good = 0;
     if ((!data && n) || (n_packets && (!packets || !units || !floor_y || !residue || !accepted)) || !n_good) return SYMGPU_ERR_ARG;
     n_threads = std::max<uint32_t>(1, std::min<uint32_t>({n_threads, 64u, std::max(1u, std::thread::hardware_concurrency()),
@@ -535,8 +559,9 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ide
     try { // no C++ exception crosses the ABI (vector / thread creation may throw)
     std::vector<symgpu_vorbis_fe*> fes(n_threads, nullptr);
     symgpu_status st = SYMGPU_OK;
-    for (uint32_t t = 0; t < n_threads && st == SYMGPU_OK; ++t) st = symgpu_vorbis_fe_create(ident, n_ident, setup, n_setup, &fes[t]);
+    for (uint32_t t = 0; t < n_threads && st == SYMGPU_OK; ++t) st = create_for(units, ident, n_ident, setup, n_setup, &fes[t]);
     if (st == SYMGPU_OK && slot < ((1u << fes[0]->ident.bs1_exp) >> 1)) st = SYMGPU_ERR_ARG;
+    if (st == SYMGPU_OK && (planes < fes[0]->ident.n_channels || planes > SYMGPU_VORBIS_MAX_CHANNELS)) st = SYMGPU_ERR_ARG;
     std::vector<uint8_t> ok(n_packets, 0);
     if (st == SYMGPU_OK) {
         std::vector<std::thread> pool;
@@ -544,8 +569,8 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ide
             pool.emplace_back([&, t] {
                 for (size_t i = t; i < n_packets; i += n_threads) {
                     if (packets[i].offset > n || packets[i].len > n - packets[i].offset) continue;
-                    ok[i] = symgpu_vorbis_fe_decode(fes[t], data + packets[i].offset, packets[i].len, slot, floor_base, units + i, floor_y + 130 * i,
-                                                    residue + 2 * size_t(slot) * i) == SYMGPU_OK;
+                    ok[i] = decode_into(fes[t], data + packets[i].offset, packets[i].len, slot, floor_base, planes, units + i,
+                                        floor_y + 65 * size_t(planes) * i, residue + size_t(planes) * slot * i) == SYMGPU_OK;
                 }
             });
         for (auto& th : pool) th.join();
@@ -568,4 +593,105 @@ extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ide
         *n_good = 0;
         return SYMGPU_ERR_LIMIT;
     }
+}
+
+}  // namespace
+
+extern "C" symgpu_status symgpu_vorbis_fe_create(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out) {
+    if (!ident || !setup || !out) return SYMGPU_ERR_ARG;
+    std::unique_ptr<symgpu_vorbis_fe> fe;
+    const symgpu_status st = open_stream(ident, n_ident, setup, n_setup, fe);
+    if (st == SYMGPU_OK && !fe->stereo) return SYMGPU_ERR_UNSUPPORTED;  // (more than two channels, or couplings the two-plane record cannot hold)
+    if (st != SYMGPU_OK) return st;
+    *out = fe.release();
+    return SYMGPU_OK;
+}
+extern "C" symgpu_status symgpu_vorbis_fe_create_mc(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, symgpu_vorbis_fe** out) {
+    if (!ident || !setup || !out) return SYMGPU_ERR_ARG;
+    std::unique_ptr<symgpu_vorbis_fe> fe;
+    const symgpu_status st = open_stream(ident, n_ident, setup, n_setup, fe);
+    if (st != SYMGPU_OK) return st;
+    *out = fe.release();
+    return SYMGPU_OK;
+}
+extern "C" void symgpu_vorbis_fe_destroy(symgpu_vorbis_fe* fe) { delete fe; }
+extern "C" void symgpu_vorbis_fe_reset(symgpu_vorbis_fe* fe) {
+    if (fe) fe->prev_block_flag = -1;
+}
+
+extern "C" symgpu_status symgpu_vorbis_fe_config(const symgpu_vorbis_fe* fe, symgpu_vorbis_stream* stream, symgpu_vorbis_floor1* floors, uint32_t* n_floors) {
+    if (!fe || !stream || !floors || !n_floors || !fe->stereo) return SYMGPU_ERR_ARG;
+    *stream = symgpu_vorbis_stream{fe->ident.bs0_exp, fe->ident.bs1_exp, fe->ident.n_channels,
+                                   uint8_t(fe->setup.mappings[fe->setup.modes[0].second].couplings.empty() ? 0 : 1)};
+    floor_records(fe, floors, n_floors);
+    return SYMGPU_OK;
+}
+extern "C" symgpu_status symgpu_vorbis_fe_config_mc(const symgpu_vorbis_fe* fe, symgpu_vorbis_stream_mc* stream, symgpu_vorbis_floor1* floors, uint32_t* n_floors) {
+    if (!fe || !stream || !floors || !n_floors) return SYMGPU_ERR_ARG;
+    std::memset(stream, 0, sizeof *stream);
+    stream->bs0_exp = fe->ident.bs0_exp, stream->bs1_exp = fe->ident.bs1_exp, stream->channels = fe->ident.n_channels;
+    const auto& couplings = fe->setup.mappings[fe->setup.modes[0].second].couplings;
+    stream->n_couplings = uint8_t(couplings.size());
+    for (size_t k = 0; k < couplings.size(); ++k) stream->magnitude_ch[k] = couplings[k].first, stream->angle_ch[k] = couplings[k].second;
+    floor_records(fe, floors, n_floors);
+    return SYMGPU_OK;
+}
+
+extern "C" symgpu_status symgpu_vorbis_fe_decode(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base,
+                                                 symgpu_vorbis_unit* unit, uint16_t* floor_y, float* residue) {
+    if (!fe || (!packet && n) || !unit || !floor_y || !residue || !fe->stereo) return SYMGPU_ERR_ARG;
+    if (slot < ((1u << fe->ident.bs1_exp) >> 1)) return SYMGPU_ERR_ARG;
+    symgpu_vorbis_unit_mc u;
+    const symgpu_status st = decode_packet(fe, packet, n, slot, floor_base, 2, &u, floor_y, residue);
+    if (st != SYMGPU_OK) return st;
+    std::memset(unit, 0, sizeof *unit);
+    unit->block_flag = u.block_flag, unit->prev_block_flag = u.prev_block_flag;
+    for (int c = 0; c < 2; ++c) unit->do_not_decode[c] = u.do_not_decode[c], unit->floor[c] = u.floor[c];
+    return SYMGPU_OK;
+}
+extern "C" symgpu_status symgpu_vorbis_fe_decode_mc(symgpu_vorbis_fe* fe, const uint8_t* packet, size_t n, uint32_t slot, uint32_t floor_base,
+                                                    uint32_t planes, symgpu_vorbis_unit_mc* unit, uint16_t* floor_y, float* residue) {
+    if (!fe || (!packet && n) || !unit || !floor_y || !residue) return SYMGPU_ERR_ARG;
+    if (slot < ((1u << fe->ident.bs1_exp) >> 1) || planes < fe->ident.n_channels || planes > SYMGPU_VORBIS_MAX_CHANNELS) return SYMGPU_ERR_ARG;
+    return decode_packet(fe, packet, n, slot, floor_base, planes, unit, floor_y, residue);
+}
+
+extern "C" symgpu_status symgpu_vorbis_fe_decode_packets(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets,
+                                                         uint32_t slot, uint32_t floor_base, symgpu_vorbis_unit* units, uint16_t* floor_y, float* residue,
+                                                         uint32_t* packet_of, size_t* n_good) {
+    if (fe && !fe->stereo) return SYMGPU_ERR_ARG;
+    return decode_packets(fe, data, n, packets, n_packets, slot, floor_base, 2, units, floor_y, residue, packet_of, n_good);
+}
+extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_mc(symgpu_vorbis_fe* fe, const uint8_t* data, size_t n, const symgpu_piece* packets,
+                                                            size_t n_packets, uint32_t slot, uint32_t floor_base, uint32_t planes,
+                                                            symgpu_vorbis_unit_mc* units, uint16_t* floor_y, float* residue, uint32_t* packet_of,
+                                                            size_t* n_good) {
+    if (fe && (planes < fe->ident.n_channels || planes > SYMGPU_VORBIS_MAX_CHANNELS)) return SYMGPU_ERR_ARG;
+    return decode_packets(fe, data, n, packets, n_packets, slot, floor_base, planes, units, floor_y, residue, packet_of, n_good);
+}
+
+extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup, const uint8_t* data,
+                                                              size_t n, const symgpu_piece* packets, size_t n_packets, uint32_t slot, uint32_t floor_base,
+                                                              symgpu_vorbis_unit* units, uint16_t* floor_y, float* residue, uint32_t* accepted, size_t* n_good,
+                                                              uint32_t n_threads) {
+    return decode_packets_jobs(ident, n_ident, setup, n_setup, data, n, packets, n_packets, slot, floor_base, 2, units, floor_y, residue, accepted,
+                               n_good, n_threads);
+}
+extern "C" symgpu_status symgpu_vorbis_fe_decode_packets_jobs_mc(const uint8_t* ident, size_t n_ident, const uint8_t* setup, size_t n_setup,
+                                                                 const uint8_t* data, size_t n, const symgpu_piece* packets, size_t n_packets,
+                                                                 uint32_t slot, uint32_t floor_base, uint32_t planes, symgpu_vorbis_unit_mc* units,
+                                                                 uint16_t* floor_y, float* residue, uint32_t* accepted, size_t* n_good,
+                                                                 uint32_t n_threads) {
+    return decode_packets_jobs(ident, n_ident, setup, n_setup, data, n, packets, n_packets, slot, floor_base, planes, units, floor_y, residue,
+                               accepted, n_good, n_threads);
+}
+
+// lib.rs:771-788 (Vorbis I 4.3.9): the output plane of Vorbis channel i
+extern "C" symgpu_status symgpu_vorbis_channel_map(uint32_t channels, uint8_t* plane_of_channel) {
+    static const uint8_t maps[SYMGPU_VORBIS_MAX_CHANNELS][SYMGPU_VORBIS_MAX_CHANNELS] = {
+        {0}, {0, 1}, {0, 2, 1}, {0, 1, 2, 3}, {0, 2, 1, 3, 4}, {0, 2, 1, 4, 5, 3}, {0, 2, 1, 5, 6, 4, 3}, {0, 2, 1, 6, 7, 4, 5, 3},
+    };
+    if (!plane_of_channel || channels < 1 || channels > SYMGPU_VORBIS_MAX_CHANNELS) return SYMGPU_ERR_ARG;
+    std::memcpy(plane_of_channel, maps[channels - 1], channels);
+    return SYMGPU_OK;
 }

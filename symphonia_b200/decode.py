@@ -5,6 +5,7 @@ import numpy as np
 
 from . import _native as nat
 from . import frontend, packetizer
+from .engine import SymgpuError
 
 
 def mpeg_audio_plan(data):
@@ -77,26 +78,49 @@ def ogg_vorbis_index(data, serial=None):
     dur, discard, _ = packetizer.vorbis_packet_durations(ident, n_modes, mask, None, heads=heads, lens=np.minimum(ln[audio], 2))
     dur, discard = dur.astype(np.int64), discard.astype(np.int64)
     trim_end = packetizer.ogg_page_end_trims(mine["page_sequence"][audio], mine["page_absgp"][audio], dur, discard).astype(np.int64)
-    fe = frontend.VorbisFrontend(ident_b, setup_b)
+    fe = open_vorbis_frontend(ident_b, setup_b)
     return dict(blob=blob, table=table[audio], ident=ident, fe=fe, discard=discard, trim_end=trim_end, headers=(ident_b, setup_b))
 
 
-def ogg_vorbis_plan(data, serial=None, index=None, out=None, slot=None, floor_base=0, threads=1):
+def open_vorbis_frontend(ident_packet, setup_packet):
+    """The stream's entropy front-end: the two-plane one (symgpu_vorbis_fe_create) for the streams it takes -- at most two channels,
+    every mapping uncoupled or coupled by the one step (0, 1) -- else the multichannel one (up to 8 channels, any coupling list)."""
+    try:
+        return frontend.VorbisFrontend(ident_packet, setup_packet)
+    except SymgpuError as e:
+        if e.status != 2:   # (SYMGPU_ERR_UNSUPPORTED: what the two-plane record cannot hold)
+            raise
+    return frontend.VorbisFrontend(ident_packet, setup_packet, mc=True)
+
+
+def vorbis_pack_map(channels):
+    """plane_of_channel for symgpu_pcm_pack_mapped_*: output channel c (the reference's order) reads Vorbis channel plane k where
+    map_vorbis_channel(channels, k) = c."""
+    return np.argsort(frontend.vorbis_channel_map(channels)).astype(np.uint8)
+
+
+def ogg_vorbis_plan(data, serial=None, index=None, out=None, slot=None, floor_base=0, threads=1, planes=None):
     """CPU half for a Vorbis-in-Ogg file: ogg_vorbis_index, then the entropy front-end (symgpu_vorbis_fe_*) over the audio packets
     -> the synthesis stage's batch and the output spans with the reader's trims.  Returns dict(stream, floors, units, floor_y, residue,
-    runs, slot, spans, channels, sample_rate, total_frames).  Packets the front-end refuses are dropped, as a caller of the reference
+    runs, slot, spans, channels, sample_rate, total_frames, mc).  Packets the front-end refuses are dropped, as a caller of the reference
     drops a DecodeError.  index / out / slot / floor_base: for `plan_files` (decode into slices of a batch whose residue rows are
-    `slot` long and whose floor tables start at `floor_base`)."""
+    `slot` long and whose floor tables start at `floor_base`).
+    A stream the two-plane front-end does not take (more than two channels, other couplings) gives a multichannel plan (mc=True): stream
+    is a VORBIS_STREAM_MC_DTYPE record, units VORBIS_UNIT_MC_DTYPE, floor_y / residue carry `planes` planes (default: the stream's
+    channels), and plane_of_channel is the channel map of the output stage (symgpu_pcm_pack_mapped_*: the reference's plane order)."""
     ix = ogg_vorbis_index(data, serial) if index is None else index
     fe, ident, discard, trim_end = ix["fe"], ix["ident"], ix["discard"], ix["trim_end"]
     slot = fe.slot if slot is None else slot
+    P = 2 if not fe.mc else (fe.channels if planes is None else int(planes))
     if threads > 1 and out is None and len(ix["table"]) >= 32:   # one long stream: its packets as independent jobs (identical output, DESIGN 10.9)
-        ju, jf, jr, keep = frontend.vorbis_decode_packets_jobs(ix["headers"][0], ix["headers"][1], ix["blob"], ix["table"], slot, floor_base, threads)
+        ju, jf, jr, keep = frontend.vorbis_decode_packets_jobs(ix["headers"][0], ix["headers"][1], ix["blob"], ix["table"], slot, floor_base, threads,
+                                                                mc=fe.mc, planes=P)
         units, fy, res = ju[keep], jf[keep], jr[keep]
     else:
-        units, fy, res, keep = fe.decode_packets(ix["blob"], ix["table"], slot=slot, floor_base=floor_base, out=out)
+        units, fy, res, keep = fe.decode_packets(ix["blob"], ix["table"], slot=slot, floor_base=floor_base, out=out, planes=P if fe.mc else None)
     n = len(units)
-    stream, floors = np.array([fe.stream], dtype=nat.VORBIS_STREAM_DTYPE), fe.floors.copy()
+    mc = fe.mc
+    stream, floors = np.array([fe.stream], dtype=nat.VORBIS_STREAM_MC_DTYPE if mc else nat.VORBIS_STREAM_DTYPE), fe.floors.copy()
     fe.close()
     bs0, bs1 = 1 << int(ident["bs0_exp"]), 1 << int(ident["bs1_exp"])
     frames = (np.where(units["prev_block_flag"] != 0, bs1, bs0) + np.where(units["block_flag"] != 0, bs1, bs0)).astype(np.int64) // 4
@@ -106,22 +130,31 @@ def ogg_vorbis_plan(data, serial=None, index=None, out=None, slot=None, floor_ba
         ts[0], te[0] = frames[0], 0   # the first packet after a reset is silenced in gapless mode (codec-vorbis lib.rs:318-322)
     left = frames - ts - te
     spans = np.zeros(n, dtype=nat.PCM_SPAN_DTYPE)
-    spans["src"] = np.arange(n, dtype=np.uint64) * (2 * slot)
+    spans["src"] = np.arange(n, dtype=np.uint64) * (P * slot)
     spans["plane_stride"], spans["frames"], spans["trim_start"], spans["trim_end"] = slot, frames, ts, te
     spans["dst_frame"] = np.concatenate([[0], np.cumsum(left)[:-1]]).astype(np.uint64) if n else 0
     total = int(left.sum())
     runs = np.zeros(1, dtype=nat.VORBIS_RUN_DTYPE)
     runs["n_packets"] = n
-    return dict(stream=stream, floors=floors, units=units, floor_y=fy, residue=res, runs=runs, slot=slot, spans=spans,
+    plan = dict(stream=stream, floors=floors, units=units, floor_y=fy, residue=res, runs=runs, slot=slot, spans=spans,
                 channels=int(ident["channels"]), sample_rate=int(ident["sample_rate"]), total_frames=total)
+    if mc:
+        plan.update(mc=True, planes=P, plane_of_channel=vorbis_pack_map(int(ident["channels"])))
+    return plan
 
 
 def decode_ogg_vorbis(engine, data, fmt=nat.FMT_S16, serial=None, threads=1):
-    """(samples [frames, channels] of `fmt`, sample_rate) of one Vorbis logical stream (mono / stereo, floor 1: what the synthesis
-    kernel takes).  Registers the stream as slot 0 of `engine` with its floors from index 0."""
+    """(samples [frames, channels] of `fmt`, sample_rate) of one Vorbis logical stream (1 to 8 channels, floor 1), channels in the
+    reference's order.  Registers the stream as slot 0 of `engine` with its floors from index 0."""
     plan = ogg_vorbis_plan(data, serial, threads=threads)
     if len(plan["units"]) == 0:
         return np.zeros((0, plan["channels"]), dtype=nat.FMT_NUMPY[fmt]), plan["sample_rate"]
+    if plan.get("mc"):
+        engine.vorbis_mc_streams_set(plan["stream"])
+        engine.vorbis_floors_set(plan["floors"])
+        pcm = engine.vorbis_mc_synth_host(plan["units"], plan["floor_y"], plan["residue"], plan["runs"], plan["planes"], plan["slot"])
+        return (engine.pcm_pack_host_mapped(pcm, plan["spans"], plan["channels"], plan["plane_of_channel"], fmt, plan["total_frames"]),
+                plan["sample_rate"])
     engine.vorbis_streams_set(plan["stream"])
     engine.vorbis_floors_set(plan["floors"])
     pcm = engine.vorbis_synth_host(plan["units"], plan["floor_y"], plan["residue"], plan["runs"], plan["slot"])
@@ -215,7 +248,8 @@ def plan_file(data):
     """CPU half of one file: dict(kind, ...) -- kind 'mp3' / 'mpa1' / 'mpa2' / 'aac' / 'vorbis'."""
     kind = sniff(data)
     if kind == "vorbis":
-        return dict(ogg_vorbis_plan(data), kind="vorbis")
+        p = ogg_vorbis_plan(data)
+        return dict(p, kind="vorbis_mc" if p.get("mc") else "vorbis")
     if kind == "aac":
         return dict(adts_aac_plan(data), kind="aac")
     if kind == "flac":
@@ -230,7 +264,10 @@ def plan_files(files, threads=None, arena=None):
     `files`, first = each member's first unit in the batch, + the arrays of that codec's synthesis entry point).  AAC files are indexed
     first and then decoded straight into their slices of the batch arrays (taken from `arena` when given: reusable staging memory);
     a file whose front-end refuses packets leaves the tail of its slice unused -- runs name what is valid.
-    A file that cannot be indexed or planned at all (an Ogg stream that is not Vorbis, more than two channels, floor 0, an ADTS channel
+    Vorbis files the two-plane synthesis takes form the batch 'vorbis'; the others (3 to 8 channels, other couplings) the batch
+    'vorbis_mc', whose arrays carry `planes` = the largest channel count among its members and whose members keep their own channel
+    maps (plane_of_channel) for the output stage.
+    A file that cannot be indexed or planned at all (an Ogg stream that is not Vorbis, more than eight channels, floor 0, an ADTS channel
     configuration outside 1 / 2, a native FLAC file, ...) does not take the others down: its plan is dict(kind="error", error=<message>)
     with no spans, it is in no batch, and pack_files returns an empty result for it."""
     import concurrent.futures
@@ -261,7 +298,8 @@ def plan_files(files, threads=None, arena=None):
         aac_units, aac_coeffs = take("aac_units", (total, 2), nat.AAC_UNIT_DTYPE), take("aac_coeffs", (total, 2, 1024), np.float32)
         vor = [i for i, k in enumerate(kinds) if k == "vorbis"]
         vindex = dict(zip(vor, pool.map(guarded(lambda i: ogg_vorbis_index(files[i])), vor)))
-        vor = [i for i in vor if i not in errors]
+        vmc = [i for i in vor if i not in errors and vindex[i]["fe"].mc]       # the multichannel batch
+        vor = [i for i in vor if i not in errors and not vindex[i]["fe"].mc]
         vstarts, vfloor, vtotal, nfl = {}, {}, 0, 0
         for i in vor:
             vstarts[i], vfloor[i] = vtotal, nfl
@@ -270,10 +308,25 @@ def plan_files(files, threads=None, arena=None):
         vslot = max([vindex[i]["fe"].slot for i in vor], default=0)
         v_units, v_fy = take("vorbis_units", (vtotal,), nat.VORBIS_UNIT_DTYPE), take("vorbis_floor_y", (vtotal, 2, 65), np.uint16)
         v_res = take("vorbis_residue", (vtotal, 2, vslot), np.float32)
+        mstarts, mfloor, mtotal, nfl = {}, {}, 0, 0
+        for i in vmc:
+            mstarts[i], mfloor[i] = mtotal, nfl
+            mtotal += len(vindex[i]["table"])
+            nfl += len(vindex[i]["fe"].floors)
+        mslot = max([vindex[i]["fe"].slot for i in vmc], default=0)
+        mplanes = max([vindex[i]["fe"].channels for i in vmc], default=1)
+        m_units = take("vorbis_mc_units", (mtotal,), nat.VORBIS_UNIT_MC_DTYPE)
+        m_fy, m_res = take("vorbis_mc_floor_y", (mtotal, mplanes, 65), np.uint16), take("vorbis_mc_residue", (mtotal, mplanes, mslot), np.float32)
 
         def plan(i):
             if i in errors:
                 return error_plan(i)
+            if kinds[i] == "vorbis" and i in mstarts:
+                a, n = mstarts[i], len(vindex[i]["table"])
+                p = ogg_vorbis_plan(files[i], index=vindex[i], out=(m_units[a:a + n], m_fy[a:a + n], m_res[a:a + n]), slot=mslot, floor_base=mfloor[i],
+                                    planes=mplanes)
+                m_units[a + len(p["units"]):a + n].view(np.uint8)[...] = 0
+                return dict(p, kind="vorbis_mc", slice_start=a)
             if kinds[i] == "vorbis":
                 a, n = vstarts[i], len(vindex[i]["table"])
                 p = ogg_vorbis_plan(files[i], index=vindex[i], out=(v_units[a:a + n], v_fy[a:a + n], v_res[a:a + n]), slot=vslot, floor_base=vfloor[i])
@@ -295,11 +348,14 @@ def plan_files(files, threads=None, arena=None):
             if kinds[i] == "vorbis" and i in vstarts:
                 a, n = vstarts[i], len(vindex[i]["table"])
                 v_units[a:a + n].view(np.uint8)[...] = 0
+            if kinds[i] == "vorbis" and i in mstarts:
+                a, n = mstarts[i], len(vindex[i]["table"])
+                m_units[a:a + n].view(np.uint8)[...] = 0
             if kinds[i] == "aac" and i in starts:
                 a, n = starts[i], len(index[i][0])
                 aac_units[a:a + n].view(np.uint8)[...] = 0
     batches = {}
-    for kind in ("mp3", "mpa1", "mpa2", "aac", "vorbis"):
+    for kind in ("mp3", "mpa1", "mpa2", "aac", "vorbis", "vorbis_mc"):
         members = [i for i, p in enumerate(plans) if p["kind"] == kind and len(p["spans"])]
         if not members:
             continue
@@ -325,15 +381,21 @@ def plan_files(files, threads=None, arena=None):
             b["units"], b["coeffs"] = aac_units, aac_coeffs
             b["tns"] = np.concatenate([plans[i]["tns"] for i in members])
             runs = np.concatenate([plans[i]["runs"] for i in members])
-        else:
+        elif kind == "vorbis":
             b["first"] = first = [plans[i]["slice_start"] for i in members]
             b["streams"] = np.concatenate([plans[i]["stream"] for i in members])
             b["floors"] = np.concatenate([vindex[i]["fe"].floors for i in vor])      # every Vorbis file's tables, in file order (floor_base)
             b["units"], b["floor_y"], b["residue"], b["slot"] = v_units, v_fy, v_res, vslot
             runs = np.concatenate([plans[i]["runs"] for i in members])
+        else:
+            b["first"] = first = [plans[i]["slice_start"] for i in members]
+            b["streams"] = np.concatenate([plans[i]["stream"] for i in members])
+            b["floors"] = np.concatenate([vindex[i]["fe"].floors for i in vmc])
+            b["units"], b["floor_y"], b["residue"], b["slot"], b["planes"] = m_units, m_fy, m_res, mslot, mplanes
+            runs = np.concatenate([plans[i]["runs"] for i in members])
         runs = runs.copy()
         runs["stream"] = np.arange(len(members))
-        runs["first_packet" if kind == "vorbis" else "first_frame"] = first
+        runs["first_packet" if kind in ("vorbis", "vorbis_mc") else "first_frame"] = first
         b["runs"] = runs
         batches[kind] = b
     return plans, batches
@@ -348,27 +410,31 @@ def _file_spans(plan, batch, k, unit_floats, plane_stride=None):
     return sp
 
 
-def pack_files(plans, batches, pcm, pack, fmt):
-    """Output stage per file: pcm[kind] = the batch's planar output, pack(pcm_slice, spans, channels, fmt, total_frames) the packer."""
+def pack_files(plans, batches, pcm, pack, fmt, pack_mapped=None):
+    """Output stage per file: pcm[kind] = the batch's planar output, pack(pcm_slice, spans, channels, fmt, total_frames) the packer,
+    pack_mapped(pcm_slice, spans, channels, plane_of_channel, fmt, total_frames) the one for files with a channel map ('vorbis_mc')."""
     out = [None] * len(plans)
     for i, p in enumerate(plans):
         if not len(p["spans"]):
             out[i] = (np.zeros((0, p["channels"]), dtype=nat.FMT_NUMPY[fmt]), p["sample_rate"])
     for kind, b in batches.items():
         flat = np.ascontiguousarray(pcm[kind]).reshape(-1)
-        per = flat.size // len(pcm[kind])          # floats per unit: two planes
+        per = flat.size // len(pcm[kind])          # floats per unit: two planes (b["planes"] in the multichannel batch)
         for k, i in enumerate(b["members"]):
             p = plans[i]
             n = len(p["spans"])
             sl = flat[b["first"][k] * per:(b["first"][k] + n) * per]
-            sp = _file_spans(p, b, k, per, per // 2)
-            out[i] = (pack(sl, sp, p["channels"], fmt, p["total_frames"]), p["sample_rate"])
+            sp = _file_spans(p, b, k, per, per // b.get("planes", 2))
+            if "plane_of_channel" in p:
+                out[i] = (pack_mapped(sl, sp, p["channels"], p["plane_of_channel"], fmt, p["total_frames"]), p["sample_rate"])
+            else:
+                out[i] = (pack(sl, sp, p["channels"], fmt, p["total_frames"]), p["sample_rate"])
     return out
 
 
 def decode_files(engine, files, fmt=nat.FMT_S16, threads=None):
     """[(samples [frames, channels], sample_rate)] for a list of MPEG audio / ADTS AAC-LC / Ogg Vorbis files: front-ends on host threads,
-    ONE synthesis launch per codec over all files (every file a stream), output stage per file.  (Re)allocates the engine's stream
+    ONE synthesis call per codec over all files (every file a stream; multichannel Vorbis files a second one), output stage per file.  (Re)allocates the engine's stream
     slots."""
     plans, batches = plan_files(files, threads)
     pcm = {}
@@ -383,11 +449,15 @@ def decode_files(engine, files, fmt=nat.FMT_S16, threads=None):
         elif kind == "aac":
             engine.aac_streams_alloc(n_streams)
             pcm[kind] = engine.aac_synth_host(b["units"], b["tns"], b["coeffs"], b["runs"])
-        else:
+        elif kind == "vorbis":
             engine.vorbis_streams_set(b["streams"])
             engine.vorbis_floors_set(b["floors"])
             pcm[kind] = engine.vorbis_synth_host(b["units"], b["floor_y"], b["residue"], b["runs"], b["slot"])
-    return pack_files(plans, batches, pcm, engine.pcm_pack_host, fmt)
+        else:   # (a context holds classic or multichannel Vorbis streams at a time: this batch runs after 'vorbis')
+            engine.vorbis_mc_streams_set(b["streams"])
+            engine.vorbis_floors_set(b["floors"])
+            pcm[kind] = engine.vorbis_mc_synth_host(b["units"], b["floor_y"], b["residue"], b["runs"], b["planes"], b["slot"])
+    return pack_files(plans, batches, pcm, engine.pcm_pack_host, fmt, engine.pcm_pack_host_mapped)
 
 
 # ---- FLAC (integer path: restoration on the GPU, samples stay int32 as in the reference's AudioBuffer<i32>) ----------------------

@@ -229,6 +229,32 @@ class Engine:
                                                   n_spans, channels, plane_stride, frames, int(fmt),
                                                   ctypes.c_void_p(out_t.data_ptr())))
 
+    def pcm_pack_host_mapped(self, pcm, spans, channels, plane_of_channel, fmt, out_frames, plane_stride=0, frames=0, n_spans=None, out=None):
+        """pcm_pack_host with a channel map: output channel c reads plane plane_of_channel[c]."""
+        pcm = np.ascontiguousarray(pcm, dtype=np.float32)
+        m = np.ascontiguousarray(plane_of_channel, dtype=np.uint8)
+        if m.size != channels:
+            raise ValueError("plane_of_channel must name one plane per output channel")
+        if spans is not None:
+            spans = np.ascontiguousarray(spans, dtype=PCM_SPAN_DTYPE)
+            n_spans = len(spans)
+        if out is None:
+            out = np.zeros((out_frames, channels), dtype=FMT_NUMPY[fmt])
+        self._check(self._lib.symgpu_pcm_pack_mapped_host(self._ctx, _np_ptr(pcm), pcm.size, _np_ptr(spans) if spans is not None else None, n_spans,
+                                                          channels, plane_stride, frames, _np_ptr(m), int(fmt), _np_ptr(out), out.nbytes))
+        return out
+
+    def pcm_pack_dev_mapped(self, pcm_t, spans_t, n_spans, channels, plane_of_channel, fmt, out_t, plane_stride=0, frames=0):
+        """Device-resident pcm_pack_host_mapped (torch CUDA tensors; the map is host memory)."""
+        assert pcm_t.is_cuda and out_t.is_cuda
+        m = np.ascontiguousarray(plane_of_channel, dtype=np.uint8)
+        if m.size != channels:
+            raise ValueError("plane_of_channel must name one plane per output channel")
+        self._check(self._lib.symgpu_pcm_pack_mapped_dev(self._ctx, ctypes.c_void_p(pcm_t.data_ptr()),
+                                                         ctypes.c_void_p(spans_t.data_ptr()) if spans_t is not None else None,
+                                                         n_spans, channels, plane_stride, frames, _np_ptr(m), int(fmt),
+                                                         ctypes.c_void_p(out_t.data_ptr())))
+
     # -- AAC --------------------------------------------------------------------------------
     def aac_streams_alloc(self, n_streams):
         self._check(self._lib.symgpu_aac_streams_alloc(self._ctx, int(n_streams)))
@@ -304,6 +330,14 @@ class Engine:
         self._check(self._lib.symgpu_vorbis_mc_synth_host(self._ctx, _np_ptr(units), _np_ptr(floor_y), _np_ptr(residue), _np_ptr(runs), len(runs), n,
                                                           C, int(slot), _np_ptr(out)))
         return out
+
+    def vorbis_mc_synth_dev(self, units_t, floor_y_t, residue_t, runs, channels, slot, pcm_t):
+        """Device-resident vorbis_mc_synth_host (torch CUDA tensors); decouples residue_t in place."""
+        runs = np.ascontiguousarray(runs, dtype=VORBIS_RUN_DTYPE)
+        n = units_t.numel() * units_t.element_size() // 32
+        self._check(self._lib.symgpu_vorbis_mc_synth_dev(
+            self._ctx, ctypes.c_void_p(units_t.data_ptr()), ctypes.c_void_p(floor_y_t.data_ptr()), ctypes.c_void_p(residue_t.data_ptr()),
+            _np_ptr(runs), len(runs), n, int(channels), int(slot), ctypes.c_void_p(pcm_t.data_ptr())))
 
     def vorbis_synth_dev(self, units_t, floor_y_t, residue_t, runs, slot, pcm_t):
         runs = np.ascontiguousarray(runs, dtype=VORBIS_RUN_DTYPE)

@@ -188,23 +188,30 @@ def flac_decode_packets(data, packets, stream_bps=0, stream_channels=0, max_bloc
 
 class VorbisFrontend:
     """One Vorbis stream's entropy front-end (codebooks, setup, previous block): identification + setup packets in, then audio
-    packets -> (unit, floor_y [2][65], residue [2][slot]), the input of Engine.vorbis_synth_host."""
+    packets -> (unit, floor_y [2][65], residue [2][slot]), the input of Engine.vorbis_synth_host.  mc=True opens the stream with
+    symgpu_vorbis_fe_create_mc (1-8 channels, any coupling list): then `stream` is a VORBIS_STREAM_MC_DTYPE record and packets come
+    out as (unit VORBIS_UNIT_MC_DTYPE, floor_y [planes][65], residue [planes][slot]), the input of Engine.vorbis_mc_synth_host;
+    `planes` (default: the stream's channel count) may be larger, so that streams of different channel counts share a batch."""
 
-    def __init__(self, ident_packet, setup_packet):
+    def __init__(self, ident_packet, setup_packet, mc=False):
         self._h = None
         self._L = nat.lib()
+        self.mc = bool(mc)
         a, b = _u8(bytes(ident_packet)), _u8(bytes(setup_packet))
         h = _vp()
-        rc = self._L.symgpu_vorbis_fe_create(_vp(a.ctypes.data), a.size, _vp(b.ctypes.data), b.size, ctypes.byref(h))
+        create = self._L.symgpu_vorbis_fe_create_mc if self.mc else self._L.symgpu_vorbis_fe_create
+        rc = create(_vp(a.ctypes.data), a.size, _vp(b.ctypes.data), b.size, ctypes.byref(h))
         if rc != 0:
-            raise SymgpuError(rc, "symgpu_vorbis_fe_create")
+            raise SymgpuError(rc, "symgpu_vorbis_fe_create_mc" if self.mc else "symgpu_vorbis_fe_create")
         self._h = h
-        stream = np.zeros(1, dtype=nat.VORBIS_STREAM_DTYPE)
+        stream = np.zeros(1, dtype=nat.VORBIS_STREAM_MC_DTYPE if self.mc else nat.VORBIS_STREAM_DTYPE)
         floors = np.zeros(64, dtype=nat.VORBIS_FLOOR1_DTYPE)
         n = ctypes.c_uint32(0)
-        self._L.symgpu_vorbis_fe_config(self._h, _vp(stream.ctypes.data), _vp(floors.ctypes.data), ctypes.byref(n))
+        config = self._L.symgpu_vorbis_fe_config_mc if self.mc else self._L.symgpu_vorbis_fe_config
+        config(self._h, _vp(stream.ctypes.data), _vp(floors.ctypes.data), ctypes.byref(n))
         self.stream, self.floors = stream[0], floors[:n.value]
         self.slot = (1 << int(self.stream["bs1_exp"])) >> 1
+        self.channels = int(self.stream["channels"])
 
     def close(self):
         if self._h:
@@ -217,43 +224,66 @@ class VorbisFrontend:
     def reset(self):
         self._L.symgpu_vorbis_fe_reset(self._h)
 
-    def decode(self, packet, slot=None, floor_base=0):
+    def _layout(self, planes):
+        if not self.mc:
+            return nat.VORBIS_UNIT_DTYPE, 2
+        return nat.VORBIS_UNIT_MC_DTYPE, self.channels if planes is None else int(planes)
+
+    def decode(self, packet, slot=None, floor_base=0, planes=None):
         slot = self.slot if slot is None else slot
+        udt, P = self._layout(planes)
         a = _u8(bytes(packet))
-        unit = np.zeros(1, dtype=nat.VORBIS_UNIT_DTYPE)
-        floor_y = np.zeros((2, 65), dtype=np.uint16)
-        residue = np.zeros((2, slot), dtype=np.float32)
-        rc = self._L.symgpu_vorbis_fe_decode(self._h, _vp(a.ctypes.data) if a.size else None, a.size, slot, floor_base, _vp(unit.ctypes.data),
-                                             _vp(floor_y.ctypes.data), _vp(residue.ctypes.data))
+        unit = np.zeros(1, dtype=udt)
+        floor_y = np.zeros((P, 65), dtype=np.uint16)
+        residue = np.zeros((P, slot), dtype=np.float32)
+        pk = (_vp(a.ctypes.data) if a.size else None, a.size, slot, floor_base)
+        outs = (_vp(unit.ctypes.data), _vp(floor_y.ctypes.data), _vp(residue.ctypes.data))
+        if self.mc:
+            rc = self._L.symgpu_vorbis_fe_decode_mc(self._h, *pk, P, *outs)
+        else:
+            rc = self._L.symgpu_vorbis_fe_decode(self._h, *pk, *outs)
         if rc != 0:
-            raise SymgpuError(rc, "symgpu_vorbis_fe_decode")
+            raise SymgpuError(rc, "symgpu_vorbis_fe_decode_mc" if self.mc else "symgpu_vorbis_fe_decode")
         return unit[0], floor_y, residue
 
-    def decode_packets(self, data, packets, slot=None, floor_base=0, out=None):
-        """All audio packets of the stream in one call (PIECE_DTYPE table over `data`): (units [g], floor_y [g,2,65], residue [g,2,slot],
-        packet_of [g]); refused packets are left out.  out = (units [>= n], floor_y [>= n,2,65], residue [>= n,2,slot]): contiguous
-        staging memory to decode into."""
+    def decode_packets(self, data, packets, slot=None, floor_base=0, out=None, planes=None):
+        """All audio packets of the stream in one call (PIECE_DTYPE table over `data`): (units [g], floor_y [g,P,65], residue [g,P,slot],
+        packet_of [g]) with P = 2 (P = planes in mc mode); refused packets are left out.  out = (units [>= n], floor_y [>= n,P,65],
+        residue [>= n,P,slot]): contiguous staging memory to decode into."""
         slot = self.slot if slot is None else slot
+        udt, P = self._layout(planes)
         a = _u8(data)
         packets = np.ascontiguousarray(packets, dtype=nat.PIECE_DTYPE)
         n = len(packets)
         if out is None:
-            units = np.zeros(n, dtype=nat.VORBIS_UNIT_DTYPE)
-            floor_y = np.zeros((n, 2, 65), dtype=np.uint16)
-            residue = np.zeros((n, 2, slot), dtype=np.float32)
+            units = np.zeros(n, dtype=udt)
+            floor_y = np.zeros((n, P, 65), dtype=np.uint16)
+            residue = np.zeros((n, P, slot), dtype=np.float32)
         else:
             units, floor_y, residue = out
-            assert all(x.flags.c_contiguous and len(x) >= n for x in out) and residue.shape[1:] == (2, slot) and residue.dtype == np.float32
-            assert units.dtype == nat.VORBIS_UNIT_DTYPE and floor_y.dtype == np.uint16 and floor_y.shape[1:] == (2, 65)
+            assert all(x.flags.c_contiguous and len(x) >= n for x in out) and residue.shape[1:] == (P, slot) and residue.dtype == np.float32
+            assert units.dtype == udt and floor_y.dtype == np.uint16 and floor_y.shape[1:] == (P, 65)
         packet_of = np.zeros(n, dtype=np.uint32)
         good = ctypes.c_size_t(0)
-        rc = self._L.symgpu_vorbis_fe_decode_packets(self._h, _vp(a.ctypes.data) if a.size else None, a.size, _vp(packets.ctypes.data), n, slot, floor_base,
-                                                     _vp(units.ctypes.data), _vp(floor_y.ctypes.data), _vp(residue.ctypes.data), _vp(packet_of.ctypes.data),
-                                                     ctypes.byref(good))
+        head = (self._h, _vp(a.ctypes.data) if a.size else None, a.size, _vp(packets.ctypes.data), n, slot, floor_base)
+        tail = (_vp(units.ctypes.data), _vp(floor_y.ctypes.data), _vp(residue.ctypes.data), _vp(packet_of.ctypes.data), ctypes.byref(good))
+        if self.mc:
+            rc = self._L.symgpu_vorbis_fe_decode_packets_mc(*head, P, *tail)
+        else:
+            rc = self._L.symgpu_vorbis_fe_decode_packets(*head, *tail)
         if rc != 0:
-            raise SymgpuError(rc, "symgpu_vorbis_fe_decode_packets")
+            raise SymgpuError(rc, "symgpu_vorbis_fe_decode_packets_mc" if self.mc else "symgpu_vorbis_fe_decode_packets")
         g = good.value
         return units[:g], floor_y[:g], residue[:g], packet_of[:g]
+
+
+def vorbis_channel_map(channels):
+    """The reference's channel order (lib.rs:771-788): out[i] = output plane of Vorbis channel i, channels 1..8."""
+    out = np.zeros(8, dtype=np.uint8)
+    rc = nat.lib().symgpu_vorbis_channel_map(int(channels), _vp(out.ctypes.data))
+    if rc != 0:
+        raise SymgpuError(rc, "symgpu_vorbis_channel_map")
+    return out[:channels]
 
 
 class AacFrontend:
@@ -364,20 +394,27 @@ def aac_decode_packets_jobs(sample_rate, channels, data, packets, tns_base=0, th
     return units, tns[:n_tns.value], coeffs
 
 
-def vorbis_decode_packets_jobs(ident_packet, setup_packet, data, packets, slot, floor_base=0, threads=4):
-    """One Vorbis stream's audio packets as independent jobs on host threads: (units [n], floor_y [n,2,65], residue [n,2,slot], accepted)
-    with outputs at their packet's index; units[accepted] etc. equal VorbisFrontend.decode_packets."""
+def vorbis_decode_packets_jobs(ident_packet, setup_packet, data, packets, slot, floor_base=0, threads=4, mc=False, planes=None):
+    """One Vorbis stream's audio packets as independent jobs on host threads: (units [n], floor_y [n,P,65], residue [n,P,slot], accepted)
+    with outputs at their packet's index; units[accepted] etc. equal VorbisFrontend(..., mc).decode_packets (P = 2, or `planes` in mc
+    mode, default the stream's channel count)."""
     a, i_, s_ = _u8(data), _u8(bytes(ident_packet)), _u8(bytes(setup_packet))
     packets = np.ascontiguousarray(packets, dtype=nat.PIECE_DTYPE)
     n = len(packets)
-    units = np.zeros(n, dtype=nat.VORBIS_UNIT_DTYPE)
-    floor_y = np.zeros((n, 2, 65), dtype=np.uint16)
-    residue = np.zeros((n, 2, slot), dtype=np.float32)
+    P = 2 if not mc else int(planes if planes is not None else (i_[11] if i_.size > 11 else 0))   # (ident byte 11: the channel count)
+    units = np.zeros(n, dtype=nat.VORBIS_UNIT_MC_DTYPE if mc else nat.VORBIS_UNIT_DTYPE)
+    floor_y = np.zeros((n, P, 65), dtype=np.uint16)
+    residue = np.zeros((n, P, slot), dtype=np.float32)
     accepted = np.zeros(n, dtype=np.uint32)
     good = ctypes.c_size_t(0)
-    rc = nat.lib().symgpu_vorbis_fe_decode_packets_jobs(_vp(i_.ctypes.data), i_.size, _vp(s_.ctypes.data), s_.size, _vp(a.ctypes.data) if a.size else None, a.size,
-                                                        _vp(packets.ctypes.data), n, int(slot), int(floor_base), _vp(units.ctypes.data), _vp(floor_y.ctypes.data),
-                                                        _vp(residue.ctypes.data), _vp(accepted.ctypes.data), ctypes.byref(good), int(threads))
+    head = (_vp(i_.ctypes.data), i_.size, _vp(s_.ctypes.data), s_.size, _vp(a.ctypes.data) if a.size else None, a.size, _vp(packets.ctypes.data), n,
+            int(slot), int(floor_base))
+    tail = (_vp(units.ctypes.data), _vp(floor_y.ctypes.data), _vp(residue.ctypes.data), _vp(accepted.ctypes.data), ctypes.byref(good), int(threads))
+    if mc:
+        rc = nat.lib().symgpu_vorbis_fe_decode_packets_jobs_mc(*head, P, *tail)
+    else:
+        rc = nat.lib().symgpu_vorbis_fe_decode_packets_jobs(*head, *tail)
     if rc != 0:
-        raise SymgpuError(rc, "symgpu_vorbis_fe_decode_packets_jobs")
+        raise SymgpuError(rc, "symgpu_vorbis_fe_decode_packets_jobs_mc" if mc else "symgpu_vorbis_fe_decode_packets_jobs")
     return units, floor_y, residue, accepted[:good.value]
+
