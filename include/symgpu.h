@@ -350,6 +350,7 @@ symgpu_status symgpu_vorbis_mc_synth_dev(symgpu_ctx* ctx, const symgpu_vorbis_un
 /* ===================================================================================================
  * Output stage (SURVEY §8f N3): planar f32 PCM -> interleaved samples of the caller's format, with
  * the decoder's gapless trim, on the device -- so that the D2H copy carries i16 instead of f32.
+ * (FLAC's integer samples have their own conversions, FromSample<i32>: see symgpu_flac_decode_*.)
  * Replaces, for the batch:
  *   AudioBuffer::trim(start, end)            symphonia-core/src/audio/buf.rs:404-433
  *     (called by the decoders at symphonia-bundle-mp3/src/decoder.rs:130-132 and
@@ -479,6 +480,27 @@ symgpu_status symgpu_flac_restore_host(symgpu_ctx* ctx, const symgpu_flac_frame*
 symgpu_status symgpu_flac_restore_dev(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
                                       const symgpu_flac_subframe* subframes, uint32_t n_subframes, int32_t* samples,
                                       size_t n_samples);
+/* Restoration as symgpu_flac_restore_*, followed by FromSample<i32> into `format` (symphonia-core/src/audio/conv.rs:514-532),
+ * interleaved: what a caller of the reference's FLAC decoder gets from AudioBuffer<i32> + copy_to_slice_interleaved::<S>.
+ *   S32  s                      S24  s >> 8 (in a 4-byte container, as the f32 output stage stores it)
+ *   S16  (s >> 16) as i16       U8   ((s as u32).wrapping_add(0x8000_0000) >> 24) as u8
+ *   F32  (s as f64 / 2^31) as f32
+ * Every rule is exact.  Frame f writes its n * channels samples from out[dst[f]] on (dst counts SAMPLES of `format`, so files with
+ * different channel counts share one call): out[dst[f] + i * channels + c] = sample i of channel c.  The restored int32 planes are
+ * not copied back.
+ * Host variant: host memory; the descriptor checks of symgpu_flac_restore_host, plus a known format, one block size for all
+ * sub-frames of a frame (SYMGPU_ERR_DECODE) and dst[f] + n * channels <= out_bytes / symgpu_sample_bytes(format)
+ * (SYMGPU_ERR_LIMIT); a refused call sends nothing to the device and leaves `out` untouched.  Otherwise `out` is rewritten in
+ * whole: samples no frame writes are zero.  `samples` is not modified.
+ * Device variant: frames, subframes, samples, dst and out in device memory, asynchronous on the context stream.  It runs the
+ * predictors in place on `samples`; n_samples bounds its reads and out_samples its writes (a frame that would leave either is not
+ * written), and the descriptors are not otherwise validated. */
+symgpu_status symgpu_flac_decode_host(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
+                                      const symgpu_flac_subframe* subframes, uint32_t n_subframes, const int32_t* samples,
+                                      size_t n_samples, const uint64_t* dst, int format, void* out, size_t out_bytes);
+symgpu_status symgpu_flac_decode_dev(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
+                                     const symgpu_flac_subframe* subframes, uint32_t n_subframes, int32_t* samples,
+                                     size_t n_samples, const uint64_t* dst, int format, void* out, size_t out_samples);
 
 /* The same synthesis fed with the QUANTISED spectra, i.e. what the Huffman stage decodes before the
  * reference turns it into f32 (read_huffman_samples: buf[i] = sign * POW43[x],

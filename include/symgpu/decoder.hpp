@@ -31,6 +31,7 @@
 #include <vector>
 
 #include "../symgpu.h"
+#include "packetizer.hpp"
 
 namespace symgpu_host {
 
@@ -58,8 +59,9 @@ inline Error map_status(symgpu_status st) { // INTEGRATION.md §3
     }
 }
 
-// Codec ids, symphonia-core/src/codecs/audio.rs:404-418.
+// Codec ids, symphonia-core/src/codecs/audio.rs:404-418, :462.
 constexpr uint32_t CODEC_ID_VORBIS = 0x1000, CODEC_ID_MP1 = 0x1004, CODEC_ID_MP2 = 0x1005, CODEC_ID_MP3 = 0x1006, CODEC_ID_AAC = 0x1007;
+constexpr uint32_t CODEC_ID_FLAC = 0x2000;
 
 struct AudioCodecParameters {
     uint32_t codec = 0;
@@ -81,10 +83,13 @@ struct Packet { // PacketRef
     const uint8_t* data = nullptr;
     size_t len = 0;
 };
-// Borrow of the decoder-owned planar f32 buffer, valid until the next call on the decoder
-// (GenericAudioBufferRef over AudioBuffer<f32>, symphonia-core/src/audio/buf.rs:68-73).
+// Borrow of the decoder-owned planar buffer, valid until the next call on the decoder (GenericAudioBufferRef over
+// AudioBuffer<f32> or AudioBuffer<i32>, symphonia-core/src/audio/buf.rs:68-73).  `format` says which planes are set.
+enum class SampleFormat { F32, S32 };
 struct AudioBufferRef {
-    const float* planes[8] = {};  // n_planes of them, in the reference's channel order
+    SampleFormat format = SampleFormat::F32;
+    const float* planes[8] = {};        // F32: n_planes of them, in the reference's channel order
+    const int32_t* planes_s32[8] = {};  // S32 (FLAC): the same for integer samples
     size_t n_planes = 0;
     size_t frames = 0;
 };
@@ -124,7 +129,7 @@ class CodecRegistry {
 // A context shared by GPU decoders (one CUDA stream).  Stream-state slots are handed out from a free list under a mutex.
 // MPEG Layer III decoders of ANY number of threads may share one context: their decode() goes through the thread-safe
 // symgpu_mp3_submit / symgpu_mp3_wait pair, which gathers the packets of all threads into shared launches.  The other decoders
-// (Layer I / II, AAC, Vorbis) still want one calling thread per context (codecs/audio.rs "Send + Sync": one call at a time).
+// (Layer I / II, AAC, Vorbis, FLAC) still want one calling thread per context (codecs/audio.rs "Send + Sync": one call at a time).
 class GpuContext {
   public:
     static Result<std::shared_ptr<GpuContext>> create(int device, uint32_t max_streams) {
@@ -495,6 +500,76 @@ class GpuVorbisDecoder final : public AudioDecoder {
     bool have_prev_ = false;
 };
 
+// FLAC decoder whose integer restoration (prediction, wasted bits, decorrelation, scaling to 32 bits) runs on the GPU (mirrors
+// FlacDecoder, symphonia-bundle-flac/src/decoder.rs:84-313).  A packet is one frame, what the reference's FLAC reader emits; the
+// frame header and the sub-frame / Rice reader run on the CPU (symgpu_flac_fe_decode_packets), the restoration as a batch of one
+// (symgpu_flac_restore_host).  The result is planar S32, as the reference's AudioBuffer<i32>.  FLAC keeps no state between packets,
+// so the decoder takes no stream slot.  finalize() does not check the MD5 of the decoded audio (INTEGRATION.md §4).
+class GpuFlacDecoder final : public AudioDecoder {
+  public:
+    static Result<std::unique_ptr<AudioDecoder>> try_new(std::shared_ptr<GpuContext> gpu, const AudioCodecParameters& p,
+                                                         const AudioDecoderOptions&) {
+        if (p.codec != CODEC_ID_FLAC) return {nullptr, {ErrorKind::Unsupported, "flac: invalid codec"}};
+        if (p.extra_data.empty()) return {nullptr, {ErrorKind::Unsupported, "flac: missing extra data"}};
+        symgpu::packet::FlacStreamInfo info{};
+        switch (symgpu::packet::flac_read_stream_info(p.extra_data.data(), p.extra_data.size(), info)) {  // StreamInfo::read
+            case symgpu::packet::Status::Ok: break;
+            case symgpu::packet::Status::EndOfStream: return {nullptr, {ErrorKind::IoError, "flac: stream information block is cut short"}};
+            case symgpu::packet::Status::Unsupported: return {nullptr, {ErrorKind::Unsupported, "flac: unsupported stream information"}};
+            default: return {nullptr, {ErrorKind::DecodeError, "flac: invalid stream information block"}};
+        }
+        AudioCodecParameters params = p;
+        params.sample_rate = info.sample_rate, params.channels = info.channels;
+        return {std::unique_ptr<AudioDecoder>(new GpuFlacDecoder(std::move(gpu), std::move(params), info)), {}};
+    }
+    void reset() override {}  // no state between packets
+    FinalizeResult finalize() override { return {}; }  // no MD5 check: has_verify stays false, also with verify = true
+    const AudioCodecParameters& codec_params() const override { return params_; }
+    Result<AudioBufferRef> decode(const Packet& packet) override {
+        frames_ = 0;  // on any error the buffer is empty
+        // decoder.rs:169-171: a block larger than the stream's largest is refused before its sub-frames are read
+        size_t at = 0;
+        while (at + 2 <= packet.len && !(packet.data[at] == 0xff && (packet.data[at + 1] & 0xfc) == 0xf8)) ++at;
+        symgpu::packet::FlacFrameHeader h{};
+        if (at + 2 <= packet.len && symgpu::packet::flac_parse_frame_header(packet.data + at, packet.len - at, h) && h.block > info_.block_max)
+            return {{}, {ErrorKind::DecodeError, "flac: allocation would overflow buffer"}};
+        const symgpu_piece piece{0, (uint32_t)packet.len, 0};
+        symgpu_flac_frame_info fi;
+        uint32_t frame_of = 0;
+        size_t n_good = 0, n_subs = 0, n_samples = 0;
+        symgpu_status st = symgpu_flac_fe_decode_packets(packet.data, packet.len, &piece, 1, info_.bits_per_sample, info_.channels, info_.block_max,
+                                                         &frame_, &fi, &frame_of, subs_, 8, samples_.data(), samples_.size(), &n_good, &n_subs,
+                                                         &n_samples);
+        if (st != SYMGPU_OK) return {{}, map_status(st)};
+        if (n_good != 1) return {{}, map_status(SYMGPU_ERR_DECODE)};
+        st = symgpu_flac_restore_host(gpu_->raw(), &frame_, 1, subs_, (uint32_t)n_subs, samples_.data(), n_samples);
+        if (st != SYMGPU_OK) return {{}, map_status(st)};
+        frames_ = fi.block_size;
+        return {last_decoded(), {}};
+    }
+    AudioBufferRef last_decoded() const override {
+        AudioBufferRef r;
+        r.format = SampleFormat::S32;
+        r.n_planes = params_.channels;
+        r.frames = frames_;
+        for (size_t c = 0; c < params_.channels; ++c)  // a frame with fewer channels than the stream leaves the others silent
+            r.planes_s32[c] = c < frame_.channels ? samples_.data() + subs_[c].offset : silence_.data();
+        return r;
+    }
+
+  private:
+    GpuFlacDecoder(std::shared_ptr<GpuContext> gpu, AudioCodecParameters p, const symgpu::packet::FlacStreamInfo& info)
+        : gpu_(std::move(gpu)), params_(std::move(p)), info_(info), samples_(size_t(info.channels) * info.block_max, 0),
+          silence_(info.block_max, 0) {}
+    std::shared_ptr<GpuContext> gpu_;
+    AudioCodecParameters params_;
+    symgpu::packet::FlacStreamInfo info_;
+    symgpu_flac_frame frame_{};
+    symgpu_flac_subframe subs_[8] = {};
+    std::vector<int32_t> samples_, silence_;
+    size_t frames_ = 0;
+};
+
 // What an application does next to symphonia::default::register_enabled_codecs (symphonia/src/lib.rs:234-255).
 inline void register_gpu_decoders(CodecRegistry& registry, std::shared_ptr<GpuContext> gpu) {
     for (uint32_t codec : {CODEC_ID_MP1, CODEC_ID_MP2, CODEC_ID_MP3})
@@ -506,6 +581,9 @@ inline void register_gpu_decoders(CodecRegistry& registry, std::shared_ptr<GpuCo
     });
     registry.register_audio_decoder_at_tier(Tier::Preferred, CODEC_ID_VORBIS, [gpu](const AudioCodecParameters& p, const AudioDecoderOptions& o) {
         return GpuVorbisDecoder::try_new(gpu, p, o);
+    });
+    registry.register_audio_decoder_at_tier(Tier::Preferred, CODEC_ID_FLAC, [gpu](const AudioCodecParameters& p, const AudioDecoderOptions& o) {
+        return GpuFlacDecoder::try_new(gpu, p, o);
     });
 }
 

@@ -193,6 +193,10 @@ def lib():
         fn = getattr(L, name)
         fn.restype = ctypes.c_int
         fn.argtypes = [vp, vp, u32, vp, u32, vp, sz]
+    for name in ("symgpu_flac_decode_host", "symgpu_flac_decode_dev"):
+        fn = getattr(L, name)
+        fn.restype = ctypes.c_int
+        fn.argtypes = [vp, vp, u32, vp, u32, vp, sz, vp, ctypes.c_int, vp, sz]
     L.symgpu_mp3_units_check.restype = ctypes.c_int
     L.symgpu_mp3_units_check.argtypes = [vp, vp, u32, u32]
     L.symgpu_aac_units_check.restype = ctypes.c_int

@@ -12,7 +12,9 @@
 // round (one coalesced request per sub-frame), the fetch of round r+1 in flight during the recurrences of round r.
 // Like the reference (decoder.rs:483-501) the predictor is instantiated for a few maximum orders with the
 // coefficients zero-padded -- exact in integer arithmetic.  flac_finish_kernel then applies the channel
-// decorrelation and the output scaling, element-wise and coalesced.
+// decorrelation and the output scaling, element-wise and coalesced.  flac_finish_pack_kernel does the same and goes on
+// to FromSample<i32> (symphonia-core/src/audio/conv.rs:514-532) and an interleaved store of the caller's format, so
+// that only the packed samples leave the device (symgpu_flac_decode_*).
 #include <cuda_runtime.h>
 
 #include <cstdint>
@@ -212,7 +214,111 @@ __global__ void __launch_bounds__(256) flac_finish_kernel(const symgpu_flac_fram
     }
 }
 
+// FromSample<i32> of conv.rs:514-532 for the output formats; every rule is exact.
+template <int FMT>
+struct FromS32;
+template <>
+struct FromS32<SYMGPU_FMT_F32> { // (s as f64 / 2^31) as f32: a power-of-two scale commutes with the rounding
+    using T = float;
+    static __device__ __forceinline__ T of(int32_t s) { return __int2float_rn(s) * 0x1p-31f; }
+};
+template <>
+struct FromS32<SYMGPU_FMT_S16> {
+    using T = int16_t;
+    static __device__ __forceinline__ T of(int32_t s) { return (int16_t)(s >> 16); }
+};
+template <>
+struct FromS32<SYMGPU_FMT_S24> { // i24::from(s >> 8), in the 4-byte container of the f32 output stage
+    using T = int32_t;
+    static __device__ __forceinline__ T of(int32_t s) { return s >> 8; }
+};
+template <>
+struct FromS32<SYMGPU_FMT_S32> {
+    using T = int32_t;
+    static __device__ __forceinline__ T of(int32_t s) { return s; }
+};
+template <>
+struct FromS32<SYMGPU_FMT_U8> {
+    using T = uint8_t;
+    static __device__ __forceinline__ T of(int32_t s) { return (uint8_t)(((uint32_t)s + 0x80000000u) >> 24); }
+};
+
+// flac_finish_kernel followed by the output stage: one CTA per frame decorrelates, scales to 32 bits, converts to FMT and
+// stores frame f interleaved at out[dst[f] ..], n * channels samples.  The restored planes are only read.  A frame whose
+// descriptors leave `samples` or `out`, or whose sub-frames disagree on the block size, is not written.
+template <int FMT>
+__global__ void __launch_bounds__(256) flac_finish_pack_kernel(const symgpu_flac_frame* __restrict__ frames, const symgpu_flac_subframe* __restrict__ subs,
+                                                               uint32_t n_subs, const int32_t* __restrict__ samples, unsigned long long n_samples,
+                                                               const unsigned long long* __restrict__ dst, void* __restrict__ out_v,
+                                                               unsigned long long out_samples) {
+    using C = FromS32<FMT>;
+    using T = typename C::T;
+    const symgpu_flac_frame fr = frames[blockIdx.x];
+    const int channels = fr.channels;
+    if (channels < 1 || channels > 8 || (unsigned long long)fr.first_subframe + channels > n_subs) return;
+    const symgpu_flac_subframe* s0 = subs + fr.first_subframe;
+    const uint32_t n = s0[0].n;
+    const unsigned long long d = dst[blockIdx.x];
+    if (d > out_samples || (unsigned long long)n * channels > out_samples - d) return;
+    for (int ch = 0; ch < channels; ++ch)
+        if (s0[ch].n != n || s0[ch].offset + n > n_samples) return;
+    const unsigned sh = fr.bits_per_sample < 32 ? 32u - fr.bits_per_sample : 0u;
+    T* __restrict__ out = static_cast<T*>(out_v) + d;
+    if (fr.assignment != SYMGPU_FLAC_INDEPENDENT && channels == 2) {
+        const int32_t* a = samples + s0[0].offset;
+        const int32_t* b = samples + s0[1].offset;
+        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
+            int32_t x = __ldg(a + i), y = __ldg(b + i);
+            if (fr.assignment == SYMGPU_FLAC_LEFT_SIDE) { // as flac_finish_kernel
+                y = wsub(x, y);
+            } else if (fr.assignment == SYMGPU_FLAC_MID_SIDE) {
+                const int32_t mid = wshl(x, 1) | (y & 1);
+                x = wadd(mid, y) >> 1;
+                y = wsub(mid, y) >> 1;
+            } else {
+                x = wadd(x, y);
+            }
+            out[2 * i] = C::of(wshl(x, sh));
+            out[2 * i + 1] = C::of(wshl(y, sh));
+        }
+    } else {
+        // one output sample per step: the stores of a warp are consecutive
+        const uint32_t total = n * (uint32_t)channels;
+        for (uint32_t j = threadIdx.x; j < total; j += blockDim.x) {
+            const uint32_t i = j / channels, c = j - i * channels;
+            out[j] = C::of(wshl(__ldg(samples + s0[c].offset + i), sh));
+        }
+    }
+}
+
+template <int FMT>
+void finish_pack_as(const symgpu_flac_frame* frames, uint32_t n_frames, const symgpu_flac_subframe* subs, uint32_t n_subs, const int32_t* samples,
+                    size_t n_samples, const uint64_t* dst, void* out, size_t out_samples, cudaStream_t stream) {
+    flac_finish_pack_kernel<FMT><<<n_frames, 256, 0, stream>>>(frames, subs, n_subs, samples, n_samples,
+                                                               reinterpret_cast<const unsigned long long*>(dst), out, out_samples);
+}
+
 } // namespace
+
+cudaError_t flac_decode_launch(const symgpu_flac_frame* frames, uint32_t n_frames, const symgpu_flac_subframe* subs, uint32_t n_subs,
+                               int32_t* samples, size_t n_samples, const uint64_t* dst, int format, void* out, size_t out_samples,
+                               cudaStream_t stream) {
+    if (format < SYMGPU_FMT_F32 || format > SYMGPU_FMT_U8) return cudaErrorInvalidValue;
+    if (n_subs) {
+        const unsigned per_block = kFlacWarps * kFlacPerWarp;
+        flac_predict_kernel<<<(n_subs + per_block - 1) / per_block, kFlacWarps * 32, 0, stream>>>(subs, n_subs, samples, n_samples);
+    }
+    if (n_frames) {
+        switch (format) {
+        case SYMGPU_FMT_F32: finish_pack_as<SYMGPU_FMT_F32>(frames, n_frames, subs, n_subs, samples, n_samples, dst, out, out_samples, stream); break;
+        case SYMGPU_FMT_S16: finish_pack_as<SYMGPU_FMT_S16>(frames, n_frames, subs, n_subs, samples, n_samples, dst, out, out_samples, stream); break;
+        case SYMGPU_FMT_S24: finish_pack_as<SYMGPU_FMT_S24>(frames, n_frames, subs, n_subs, samples, n_samples, dst, out, out_samples, stream); break;
+        case SYMGPU_FMT_S32: finish_pack_as<SYMGPU_FMT_S32>(frames, n_frames, subs, n_subs, samples, n_samples, dst, out, out_samples, stream); break;
+        default: finish_pack_as<SYMGPU_FMT_U8>(frames, n_frames, subs, n_subs, samples, n_samples, dst, out, out_samples, stream); break;
+        }
+    }
+    return cudaGetLastError();
+}
 
 cudaError_t flac_launch(const symgpu_flac_frame* frames, uint32_t n_frames, const symgpu_flac_subframe* subs, uint32_t n_subs,
                         int32_t* samples, size_t n_samples, cudaStream_t stream) {

@@ -588,12 +588,12 @@ symgpu_status symgpu_flac_restore_dev(symgpu_ctx* ctx, const symgpu_flac_frame* 
     return SYMGPU_OK;
 }
 
-symgpu_status symgpu_flac_restore_host(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
-                                       const symgpu_flac_subframe* subframes, uint32_t n_subframes, int32_t* samples,
-                                       size_t n_samples) {
-    if (!ctx || !frames || !subframes || !samples) return SYMGPU_ERR_ARG;
-    // What read_subframe / decode_linear / decode_fixed_linear refuse (decoder.rs:335-347, :429-431, :456-474,
-    // :503-505) is refused here; the kernels additionally never leave the buffer.
+} // extern "C"
+
+// What read_subframe / decode_linear / decode_fixed_linear refuse (decoder.rs:335-347, :429-431, :456-474,
+// :503-505) is refused here; the kernels additionally never leave the buffer.
+static symgpu_status flac_descriptors_check(const symgpu_flac_frame* frames, uint32_t n_frames, const symgpu_flac_subframe* subframes,
+                                            uint32_t n_subframes, size_t n_samples) {
     for (uint32_t k = 0; k < n_subframes; ++k) {
         const symgpu_flac_subframe& sf = subframes[k];
         if (sf.n == 0 || sf.offset > n_samples || sf.n > n_samples - sf.offset) return SYMGPU_ERR_ARG;
@@ -611,12 +611,23 @@ symgpu_status symgpu_flac_restore_host(symgpu_ctx* ctx, const symgpu_flac_frame*
             (fr.channels != 2 || subframes[fr.first_subframe].n != subframes[fr.first_subframe + 1].n))
             return SYMGPU_ERR_DECODE;
     }
+    return SYMGPU_OK;
+}
+
+extern "C" {
+
+symgpu_status symgpu_flac_restore_host(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
+                                       const symgpu_flac_subframe* subframes, uint32_t n_subframes, int32_t* samples,
+                                       size_t n_samples) {
+    if (!ctx || !frames || !subframes || !samples) return SYMGPU_ERR_ARG;
+    symgpu_status s = flac_descriptors_check(frames, n_frames, subframes, n_subframes, n_samples);
+    if (s != SYMGPU_OK) return s;
     if (n_frames == 0 && n_subframes == 0) return SYMGPU_OK;
     DeviceGuard guard(ctx->device);
     const size_t sample_bytes = (n_samples * sizeof(int32_t) + 255) & ~(size_t)255;
     const size_t sub_bytes = ((size_t)n_subframes * sizeof(symgpu_flac_subframe) + 255) & ~(size_t)255;
     const size_t frame_bytes = (size_t)n_frames * sizeof(symgpu_flac_frame);
-    symgpu_status s = ensure_stage(ctx, sample_bytes + sub_bytes + frame_bytes);
+    s = ensure_stage(ctx, sample_bytes + sub_bytes + frame_bytes);
     if (s != SYMGPU_OK) return s;
     char* base = static_cast<char*>(ctx->d_stage);
     int32_t* d_samples = reinterpret_cast<int32_t*>(base);
@@ -628,6 +639,63 @@ symgpu_status symgpu_flac_restore_host(symgpu_ctx* ctx, const symgpu_flac_frame*
     s = symgpu_flac_restore_dev(ctx, d_frames, n_frames, d_subs, n_subframes, d_samples, n_samples);
     if (s != SYMGPU_OK) return s;
     CU(ctx, cudaMemcpyAsync(samples, d_samples, n_samples * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return SYMGPU_OK;
+}
+
+// ---- FLAC restoration + output stage (FromSample<i32>, conv.rs:514-532) -------------------------------------------------------
+symgpu_status symgpu_flac_decode_dev(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
+                                     const symgpu_flac_subframe* subframes, uint32_t n_subframes, int32_t* samples,
+                                     size_t n_samples, const uint64_t* dst, int format, void* out, size_t out_samples) {
+    if (!ctx || !frames || !subframes || !samples || !dst || !out) return SYMGPU_ERR_ARG;
+    if (symgpu_sample_bytes(format) == 0) return SYMGPU_ERR_ARG;
+    if (n_frames == 0 && n_subframes == 0) return SYMGPU_OK;
+    DeviceGuard guard(ctx->device);
+    CU(ctx, flac_decode_launch(frames, n_frames, subframes, n_subframes, samples, n_samples, dst, format, out, out_samples, ctx->stream));
+    ctx->launches += (n_subframes ? 1 : 0) + (n_frames ? 1 : 0);
+    return SYMGPU_OK;
+}
+
+symgpu_status symgpu_flac_decode_host(symgpu_ctx* ctx, const symgpu_flac_frame* frames, uint32_t n_frames,
+                                      const symgpu_flac_subframe* subframes, uint32_t n_subframes, const int32_t* samples,
+                                      size_t n_samples, const uint64_t* dst, int format, void* out, size_t out_bytes) {
+    if (!ctx || !frames || !subframes || !samples || !dst || !out) return SYMGPU_ERR_ARG;
+    const size_t sb = symgpu_sample_bytes(format);
+    if (sb == 0) return SYMGPU_ERR_ARG;
+    symgpu_status s = flac_descriptors_check(frames, n_frames, subframes, n_subframes, n_samples);
+    if (s != SYMGPU_OK) return s;
+    // Interleaving needs one block size per frame, and every frame's samples inside `out`.
+    const uint64_t out_samples = out_bytes / sb;
+    for (uint32_t f = 0; f < n_frames; ++f) {
+        const symgpu_flac_frame& fr = frames[f];
+        const uint32_t n = subframes[fr.first_subframe].n;
+        for (uint32_t c = 1; c < fr.channels; ++c)
+            if (subframes[fr.first_subframe + c].n != n) return SYMGPU_ERR_DECODE;
+        if (dst[f] > out_samples || (uint64_t)n * fr.channels > out_samples - dst[f]) return SYMGPU_ERR_LIMIT;
+    }
+    if (n_frames == 0 && n_subframes == 0) return SYMGPU_OK;
+    DeviceGuard guard(ctx->device);
+    const size_t sample_bytes = (n_samples * sizeof(int32_t) + 255) & ~(size_t)255;
+    const size_t sub_bytes = ((size_t)n_subframes * sizeof(symgpu_flac_subframe) + 255) & ~(size_t)255;
+    const size_t frame_bytes = ((size_t)n_frames * sizeof(symgpu_flac_frame) + 255) & ~(size_t)255;
+    const size_t dst_bytes = ((size_t)n_frames * sizeof(uint64_t) + 255) & ~(size_t)255;
+    const size_t packed = out_samples * sb;
+    s = ensure_stage(ctx, sample_bytes + sub_bytes + frame_bytes + dst_bytes + packed);
+    if (s != SYMGPU_OK) return s;
+    char* base = static_cast<char*>(ctx->d_stage);
+    int32_t* d_samples = reinterpret_cast<int32_t*>(base);
+    symgpu_flac_subframe* d_subs = reinterpret_cast<symgpu_flac_subframe*>(base + sample_bytes);
+    symgpu_flac_frame* d_frames = reinterpret_cast<symgpu_flac_frame*>(base + sample_bytes + sub_bytes);
+    uint64_t* d_dst = reinterpret_cast<uint64_t*>(base + sample_bytes + sub_bytes + frame_bytes);
+    void* d_out = base + sample_bytes + sub_bytes + frame_bytes + dst_bytes;
+    CU(ctx, cudaMemcpyAsync(d_samples, samples, n_samples * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(d_subs, subframes, (size_t)n_subframes * sizeof(symgpu_flac_subframe), cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(d_frames, frames, (size_t)n_frames * sizeof(symgpu_flac_frame), cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(d_dst, dst, (size_t)n_frames * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemsetAsync(d_out, 0, packed, ctx->stream)); // samples no frame writes are zero
+    s = symgpu_flac_decode_dev(ctx, d_frames, n_frames, d_subs, n_subframes, d_samples, n_samples, d_dst, format, d_out, out_samples);
+    if (s != SYMGPU_OK) return s;
+    CU(ctx, cudaMemcpyAsync(out, d_out, packed, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return SYMGPU_OK;
 }

@@ -238,14 +238,14 @@ def sniff(data):
     if head == b"OggS":
         return "vorbis"
     if head == b"fLaC":
-        return "flac"  # the integer path has its own entry point (decode_flac); plan_files reports it as an error for that file
+        return "flac"  # the integer path: restoration + FromSample<i32> on the device, not the f32 synthesis batches
     if len(head) >= 2 and head[0] == 0xFF and (head[1] & 0xF6) == 0xF0:
         return "aac"
     return "mpa"
 
 
 def plan_file(data):
-    """CPU half of one file: dict(kind, ...) -- kind 'mp3' / 'mpa1' / 'mpa2' / 'aac' / 'vorbis'."""
+    """CPU half of one file: dict(kind, ...) -- kind 'mp3' / 'mpa1' / 'mpa2' / 'aac' / 'vorbis' / 'vorbis_mc' / 'flac' (flac_plan)."""
     kind = sniff(data)
     if kind == "vorbis":
         p = ogg_vorbis_plan(data)
@@ -253,7 +253,7 @@ def plan_file(data):
     if kind == "aac":
         return dict(adts_aac_plan(data), kind="aac")
     if kind == "flac":
-        raise ValueError("native FLAC goes through decode_flac (integer samples), not through the f32 synthesis batches")
+        return dict(flac_plan(data), kind="flac")
     layer, payload, runs, spans, rate, channels, total = mpeg_audio_plan(data)
     return dict(kind={1: "mpa1", 2: "mpa2", 3: "mp3"}[layer], payload=payload, runs=runs, spans=spans, sample_rate=rate, channels=channels, total_frames=total)
 
@@ -267,9 +267,13 @@ def plan_files(files, threads=None, arena=None):
     Vorbis files the two-plane synthesis takes form the batch 'vorbis'; the others (3 to 8 channels, other couplings) the batch
     'vorbis_mc', whose arrays carry `planes` = the largest channel count among its members and whose members keep their own channel
     maps (plane_of_channel) for the output stage.
+    Native FLAC files are planned by flac_plan (kind 'flac') and form the batch 'flac', the input of ONE symgpu_flac_decode_host call:
+    frames, subframes and samples concatenated (first_subframe and the sub-frame offsets re-based), dst placing every file's output in
+    its own [total_frames, channels] region of one flat buffer of out_samples samples, out_first[k] = where member k's region starts.
+    FLAC plans have no spans: pack_files leaves them alone and decode_files fills them in from that call.
     A file that cannot be indexed or planned at all (an Ogg stream that is not Vorbis, more than eight channels, floor 0, an ADTS channel
-    configuration outside 1 / 2, a native FLAC file, ...) does not take the others down: its plan is dict(kind="error", error=<message>)
-    with no spans, it is in no batch, and pack_files returns an empty result for it."""
+    configuration outside 1 / 2, a FLAC file without a valid STREAMINFO, ...) does not take the others down: its plan is
+    dict(kind="error", error=<message>) with no spans, it is in no batch, and pack_files returns an empty result for it."""
     import concurrent.futures
     import os
     kinds = [sniff(f) for f in files]
@@ -333,6 +337,8 @@ def plan_files(files, threads=None, arena=None):
                 tail = v_units[a + len(p["units"]):a + n].view(np.uint8)
                 tail[...] = 0
                 return dict(p, kind="vorbis", slice_start=a)
+            if kinds[i] == "flac":
+                return dict(flac_plan(files[i]), kind="flac")
             if kinds[i] != "aac":
                 return plan_file(files[i])
             a, n = starts[i], len(index[i][0])
@@ -398,6 +404,20 @@ def plan_files(files, threads=None, arena=None):
         runs["first_packet" if kind in ("vorbis", "vorbis_mc") else "first_frame"] = first
         b["runs"] = runs
         batches[kind] = b
+    members = [i for i, p in enumerate(plans) if p["kind"] == "flac" and len(p["frames"])]
+    if members:
+        frames, subs, dst, out_first = [], [], [], []
+        n_sub = n_smp = out_at = 0
+        for i in members:
+            p = plans[i]
+            f, s = p["frames"].copy(), p["subframes"].copy()
+            f["first_subframe"] += n_sub
+            s["offset"] += np.uint64(n_smp)
+            frames.append(f), subs.append(s), dst.append(flac_dst(p, out_at)), out_first.append(out_at)
+            n_sub, n_smp, out_at = n_sub + len(s), n_smp + len(p["samples"]), out_at + p["total_frames"] * p["channels"]
+        batches["flac"] = dict(members=members, out_first=out_first, out_samples=out_at, frames=np.concatenate(frames),
+                               subframes=np.concatenate(subs), samples=np.concatenate([plans[i]["samples"] for i in members]),
+                               dst=np.concatenate(dst))
     return plans, batches
 
 
@@ -412,12 +432,15 @@ def _file_spans(plan, batch, k, unit_floats, plane_stride=None):
 
 def pack_files(plans, batches, pcm, pack, fmt, pack_mapped=None):
     """Output stage per file: pcm[kind] = the batch's planar output, pack(pcm_slice, spans, channels, fmt, total_frames) the packer,
-    pack_mapped(pcm_slice, spans, channels, plane_of_channel, fmt, total_frames) the one for files with a channel map ('vorbis_mc')."""
+    pack_mapped(pcm_slice, spans, channels, plane_of_channel, fmt, total_frames) the one for files with a channel map ('vorbis_mc').
+    FLAC plans and the 'flac' batch are not packed here (their output stage is part of symgpu_flac_decode_*): their entries stay None."""
     out = [None] * len(plans)
     for i, p in enumerate(plans):
-        if not len(p["spans"]):
+        if p["kind"] != "flac" and not len(p["spans"]):
             out[i] = (np.zeros((0, p["channels"]), dtype=nat.FMT_NUMPY[fmt]), p["sample_rate"])
     for kind, b in batches.items():
+        if kind == "flac":
+            continue
         flat = np.ascontiguousarray(pcm[kind]).reshape(-1)
         per = flat.size // len(pcm[kind])          # floats per unit: two planes (b["planes"] in the multichannel batch)
         for k, i in enumerate(b["members"]):
@@ -433,14 +456,17 @@ def pack_files(plans, batches, pcm, pack, fmt, pack_mapped=None):
 
 
 def decode_files(engine, files, fmt=nat.FMT_S16, threads=None):
-    """[(samples [frames, channels], sample_rate)] for a list of MPEG audio / ADTS AAC-LC / Ogg Vorbis files: front-ends on host threads,
-    ONE synthesis call per codec over all files (every file a stream; multichannel Vorbis files a second one), output stage per file.  (Re)allocates the engine's stream
-    slots."""
+    """[(samples [frames, channels], sample_rate)] for a list of MPEG audio / ADTS AAC-LC / Ogg Vorbis / native FLAC files: front-ends on
+    host threads, ONE synthesis call per codec over all files (every file a stream; multichannel Vorbis files a second one), output stage
+    per file.  All FLAC files share one symgpu_flac_decode_host call (restoration, FromSample<i32> into `fmt`, interleaving), whose
+    output is cut per file.  (Re)allocates the engine's stream slots."""
     plans, batches = plan_files(files, threads)
-    pcm = {}
+    pcm, flac = {}, None
     for kind, b in batches.items():
         n_streams = len(b["members"])
-        if kind == "mp3":
+        if kind == "flac":
+            flac = engine.flac_decode_host(b["frames"], b["subframes"], b["samples"], b["dst"], fmt, b["out_samples"])
+        elif kind == "mp3":
             engine.mp3_streams_alloc(n_streams)
             pcm[kind] = engine.mp3_synth_host_quantized(b["units"], b["quant"], b["runs"])
         elif kind in ("mpa1", "mpa2"):
@@ -457,7 +483,14 @@ def decode_files(engine, files, fmt=nat.FMT_S16, threads=None):
             engine.vorbis_mc_streams_set(b["streams"])
             engine.vorbis_floors_set(b["floors"])
             pcm[kind] = engine.vorbis_mc_synth_host(b["units"], b["floor_y"], b["residue"], b["runs"], b["planes"], b["slot"])
-    return pack_files(plans, batches, pcm, engine.pcm_pack_host, fmt, engine.pcm_pack_host_mapped)
+    out = pack_files(plans, batches, pcm, engine.pcm_pack_host, fmt, engine.pcm_pack_host_mapped)
+    at = dict(zip(batches["flac"]["members"], batches["flac"]["out_first"])) if flac is not None else {}
+    for i, p in enumerate(plans):
+        if p["kind"] == "flac":
+            n, ch = (p["total_frames"], p["channels"]) if i in at else (0, p["channels"])
+            region = flac[at[i]:at[i] + n * ch] if i in at else np.zeros(0, dtype=nat.FMT_NUMPY[fmt])
+            out[i] = (region.reshape(n, ch), p["sample_rate"])
+    return out
 
 
 # ---- FLAC (integer path: restoration on the GPU, samples stay int32 as in the reference's AudioBuffer<i32>) ----------------------
@@ -489,10 +522,22 @@ def flac_interleave(plan, restored):
     return out
 
 
-def decode_flac(engine, data):
-    """(samples [frames, channels] int32 scaled to 32 bits as the reference's FLAC decoder leaves them, sample_rate)."""
+def flac_dst(plan, base=0):
+    """Output position (in samples) of every frame of a FLAC plan for symgpu_flac_decode_*: the frames back to back from `base`, each
+    n * channels samples, so that the plan's output is one [total_frames, channels] region."""
+    frames = plan["frames"]
+    n = plan["subframes"]["n"][frames["first_subframe"]].astype(np.uint64) * frames["channels"].astype(np.uint64)
+    return (np.uint64(base) + np.concatenate([[0], np.cumsum(n)[:-1]])).astype(np.uint64) if len(frames) else np.zeros(0, dtype=np.uint64)
+
+
+def decode_flac(engine, data, fmt=None):
+    """(samples [frames, channels], sample_rate) of a native FLAC file.  fmt None: int32 scaled to 32 bits as the reference's FLAC
+    decoder leaves them (AudioBuffer<i32>); else samples of that FMT_* by FromSample<i32> (conv.rs:514-532).  Restoration, conversion and
+    interleaving run in one device call (symgpu_flac_decode_host; None is its identity conversion FMT_S32)."""
     plan = flac_plan(data)
+    code = nat.FMT_S32 if fmt is None else fmt
+    out = np.zeros((plan["total_frames"], plan["channels"]), dtype=nat.FMT_NUMPY[code])
     if len(plan["frames"]) == 0:
-        return np.zeros((0, plan["channels"]), dtype=np.int32), plan["sample_rate"]
-    restored = engine.flac_restore_host(plan["frames"], plan["subframes"], plan["samples"].copy())
-    return flac_interleave(plan, restored), plan["sample_rate"]
+        return out, plan["sample_rate"]
+    engine.flac_decode_host(plan["frames"], plan["subframes"], plan["samples"], flac_dst(plan), code, out=out)
+    return out, plan["sample_rate"]

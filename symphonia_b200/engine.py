@@ -206,6 +206,35 @@ class Engine:
                                                       ctypes.c_void_p(subframes_t.data_ptr()), n_subframes,
                                                       ctypes.c_void_p(samples_t.data_ptr()), samples_t.numel()))
 
+    def flac_decode_host(self, frames, subframes, samples, dst, fmt, out_samples=None, out=None):
+        """Restoration + FromSample<i32> into `fmt` (FMT_*), interleaved: frame f's n * channels samples at flat index dst[f] of
+        the result, a 1-D array of out_samples samples of `fmt` (or `out`, any shape).  `samples` (int32) is left as it is."""
+        from ._native import FLAC_FRAME_DTYPE, FLAC_SUBFRAME_DTYPE
+        frames = np.ascontiguousarray(frames, dtype=FLAC_FRAME_DTYPE)
+        subframes = np.ascontiguousarray(subframes, dtype=FLAC_SUBFRAME_DTYPE)
+        samples = np.ascontiguousarray(samples, dtype=np.int32)
+        dst = np.ascontiguousarray(dst, dtype=np.uint64)
+        if len(dst) != len(frames):
+            raise ValueError("dst must hold one output position per frame")
+        if out is None:
+            out = np.empty(int(out_samples), dtype=FMT_NUMPY[fmt])
+        assert out.flags.c_contiguous
+        self._check(self._lib.symgpu_flac_decode_host(self._ctx, _np_ptr(frames), len(frames), _np_ptr(subframes), len(subframes),
+                                                      _np_ptr(samples), samples.size, _np_ptr(dst), int(fmt), _np_ptr(out), out.nbytes))
+        return out
+
+    def flac_decode_dev(self, frames_t, n_frames, subframes_t, n_subframes, samples_t, dst_t, fmt, out_t, out_samples=None):
+        """Device-resident flac_decode_host (torch CUDA tensors; dst_t int64 / uint64 per frame).  Runs the predictors in place on
+        samples_t; out_samples defaults to what out_t holds in samples of `fmt`."""
+        assert frames_t.is_cuda and subframes_t.is_cuda and samples_t.is_cuda and dst_t.is_cuda and out_t.is_cuda
+        if out_samples is None:
+            out_samples = out_t.numel() * out_t.element_size() // np.dtype(FMT_NUMPY[fmt]).itemsize
+        self._check(self._lib.symgpu_flac_decode_dev(self._ctx, ctypes.c_void_p(frames_t.data_ptr()), n_frames,
+                                                     ctypes.c_void_p(subframes_t.data_ptr()), n_subframes,
+                                                     ctypes.c_void_p(samples_t.data_ptr()), samples_t.numel(),
+                                                     ctypes.c_void_p(dst_t.data_ptr()), int(fmt),
+                                                     ctypes.c_void_p(out_t.data_ptr()), int(out_samples)))
+
     # -- output stage -------------------------------------------------------------------------
     def pcm_pack_host(self, pcm, spans, channels, fmt, out_frames, plane_stride=0, frames=0, n_spans=None, out=None):
         """Trim + interleave + convert planar f32 `pcm` (any shape, flat indexing) into [out_frames, channels]
