@@ -106,6 +106,13 @@ def main():
         ok = all(a == b[:len(a)] and not any(b[len(a):]) for a, b in zip(r, mm)) and len(r) == len(mm)
         print(f"{rname:28s} {'OK' if ok else 'MISMATCH'}")
         bad += 0 if ok else 1
+    # the mixed-block switch points and band counts (tests/_mp3_f64_model.py reads them from the header too)
+    ref_switch = [int(x) for x in re.search(r"SFB_MIXED_SWITCH_POINT: \[usize; 9\] = \[(.*?)\];", csrc).group(1).split(",")]
+    my_count, my_switch = ([int(x) for x in re.search(name + r"\[9\] = \{(.*?)\};", hdr).group(1).split(",")]
+                           for name in ("kMixedCount", "kMixedSwitch"))
+    ok = my_switch == ref_switch and my_count == [len(r) for r in ref_tab("SFB_MIXED_BANDS")]
+    print(f"{'SFB_MIXED_SWITCH_POINT':28s} {'OK' if ok else 'MISMATCH'}")
+    bad += 0 if ok else 1
     print("FAILED" if bad else "ALL CONSTANTS MATCH THE REFERENCE")
     return 1 if bad else 0
 
